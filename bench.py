@@ -22,7 +22,7 @@ Printed JSON (one line, rank 0).  Besides the contract's keys:
   cpu_baseline the reference's own modules (transpiled, oracle/_ref) on all host cores: persistent thread pool,
                instance + precompute once per size outside the timed region, memcpy-in + transform per row
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 """
 from __future__ import annotations
 
@@ -306,6 +306,46 @@ def run_reference(args):
 # --------------------------------------------------------------------------------------------
 # our arm
 # --------------------------------------------------------------------------------------------
+DUMP_FLOATS = 1 << 18       # floats per dumped array (1 MiB): 9 sizes x 4 planes = 36 MiB in all
+
+
+def dump_outputs(out_dir, steps, step, seed_input, a, b):
+    """--dump-outputs: writes what the last of the `steps` timed headline steps returned at each size -- the forward
+    spectrum and the inverse's result, split re/im planes, a fixed seeded sample of rows of each -- as
+    <out_dir>/<name>.npy (float32).  The timed steps start from the seeded input and the kernels are deterministic, so
+    replaying steps - 1 steps and capturing the next one reproduces the last timed step; the replay is checked bit for
+    bit against the state the timed steps left (at the largest size, whose outputs the step does not overwrite)."""
+    import numpy as np
+    import torch
+    pick = np.random.default_rng(20250)
+    rows = {}
+    for n in SIZES:
+        batch = GIB // (8 * n)
+        rows[n] = torch.as_tensor(np.sort(pick.choice(batch, min(batch, DUMP_FLOATS // n), replace=False)),
+                                  device=a[0].device)
+
+    def take(n, planes):
+        return [p.view(-1, n).index_select(0, rows[n]).cpu().numpy() for p in planes]
+
+    out = {}
+
+    def capture(n, direction, re, im):
+        out[f"c2c_f32_split_n{n}_{direction}_re"], out[f"c2c_f32_split_n{n}_{direction}_im"] = take(n, (re, im))
+
+    n = SIZES[-1]
+    timed = take(n, b) + take(n, a)
+    seed_input()
+    for _ in range(steps - 1):
+        step()
+    step(capture=capture)
+    replayed = [out[f"c2c_f32_split_n{n}_{d}_{p}"] for d in ("forward", "inverse") for p in ("re", "im")]
+    assert all(np.array_equal(x, y) for x, y in zip(timed, replayed)), "replayed last step differs from the timed one"
+    assert sum(x.nbytes for x in out.values()) <= 64 * 10**6
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), x)
+
+
 def run_ours(args):
     import ctypes
     import numpy as np
@@ -364,8 +404,11 @@ def run_ours(args):
     b_ptr = a_ptr + GIB + SLACK
     A32 = arena[: GIB].view(torch.float32)
     g = torch.Generator(device=dev)
-    g.manual_seed(1234 + rank)
-    A32.uniform_(-1, 1, generator=g)
+
+    def seed_input():
+        g.manual_seed(1234 + rank)
+        A32.uniform_(-1, 1, generator=g)
+    seed_input()
     nfloat = GIB // 8
     a_re, a_im = A32[:nfloat], A32[nfloat:]
     Bv = arena[GIB + SLACK: 2 * GIB + SLACK].view(torch.float32)
@@ -377,14 +420,18 @@ def run_ours(args):
     A = (a_re.data_ptr(), a_im.data_ptr())
     B = (b_re.data_ptr(), b_im.data_ptr())
 
-    def step(events=None):
+    def step(events=None, capture=None):
         for i, n in enumerate(SIZES):
             if events is not None:
                 events[2 * i].record(stream)
             plans[n].exec_device(C.FORWARD, A, B, sptr)       # A -> B
+            if capture is not None:
+                capture(n, "forward", b_re, b_im)
             if events is not None:
                 events[2 * i + 1].record(stream)
             plans[n].exec_device(C.INVERSE, B, A, sptr)       # B -> A (round trip restores the data)
+            if capture is not None:
+                capture(n, "inverse", a_re, a_im)
         if events is not None:
             events[2 * len(SIZES)].record(stream)
 
@@ -399,11 +446,12 @@ def run_ours(args):
         step()
     barrier()
     t_w = time.perf_counter()
-    extra_warm = 0
     while time.perf_counter() - t_w < 0.75:
         step()
         torch.cuda.synchronize()
-        extra_warm += 1
+    # the warm-up made a wall-clock-dependent number of round trips over A: the timed steps start again from the seeded
+    # input, so that they compute the same values in every run with the same arguments
+    seed_input()
     launches0 = lib.wfb_kernel_launch_count()
     K = args.steps
     evs = [[torch.cuda.Event(enable_timing=True) for _ in range(2 * len(SIZES) + 1)] for _ in range(K)]
@@ -419,10 +467,13 @@ def run_ours(args):
     elapsed_ms = t_begin.elapsed_time(t_end)
     clocks = sampler.stop() if sampler else None
     # the round trips must have restored the input: proof the timed launches did the work.  f32 rounding
-    # accumulates over the ~10^3 fft->ifft round trips of a run, so the bound scales with their number ...
-    trips = len(SIZES) * (K + warm + extra_warm)
+    # accumulates over the fft->ifft round trips since the input was seeded (those of the timed steps), so the bound
+    # scales with their number ...
+    trips = len(SIZES) * K
     drift = float((a_re[: 1 << 20] - ref_re).abs().max())
     assert drift < max(1e-3, 4e-6 * trips), f"round-trip drift {drift} after {trips} round trips"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, K, step, seed_input, (a_re, a_im), (b_re, b_im))
     # ... and one fresh step on pristine data must come back within the reference's own round-trip tolerance
     a_re[: 1 << 20] = ref_re
     a_im[: 1 << 20] = ref_im
@@ -881,7 +932,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sharded-e2e", action="store_true", help="skip the one-process configs[4] end-to-end leg (N > 1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a seeded sample of what the last timed headline step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU headline path (--impl ours)")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if not (args.impl == "ours" and args.gpus > 1 and world == 1):      # (the torchrun re-launch prints through its ranks)
         quiet_stdout()
@@ -892,6 +949,8 @@ def main():
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}",
                "--master-addr", "127.0.0.1", "--master-port", "29541", __file__, "--gpus", str(args.gpus),
                "--steps", str(args.steps), "--warmup", str(args.warmup)]
+        if args.dump_outputs:
+            cmd += ["--dump-outputs", args.dump_outputs]
         return subprocess.call(cmd)
     return run_ours(args)
 

@@ -31,15 +31,24 @@ _c_f32p = ctypes.POINTER(ctypes.c_float)
 _c_f64p = ctypes.POINTER(ctypes.c_double)
 
 
+def reference_modules() -> Path | None:
+    """``modules/`` of the wat-fft checkout named by $WATFFT_REFERENCE, or None when it is not set."""
+    ref = os.environ.get("WATFFT_REFERENCE")
+    return Path(ref) / "modules" if ref else None
+
+
 def build(force: bool = False) -> None:
-    """Compile the restatement and, when /root/reference is present, libwatref."""
+    """Compile the restatement and, when $WATFFT_REFERENCE names a wat-fft checkout, libwatref."""
     src = HERE / "watfft_oracle.c"
     if force or not ORACLE_SO.exists() or ORACLE_SO.stat().st_mtime < src.stat().st_mtime:
         subprocess.check_call(["make", "-C", str(HERE), "libwatfft_oracle.so"], stdout=subprocess.DEVNULL)
-    if Path("/root/reference/modules").is_dir():
+    mods = reference_modules()
+    if mods is not None:
+        if not mods.is_dir():
+            raise FileNotFoundError(f"WATFFT_REFERENCE: {mods} is not a directory")
         newest = max(p.stat().st_mtime for p in [HERE / "wat2c.py", HERE / "watref_threads.c"])
         if force or not WATREF_SO.exists() or WATREF_SO.stat().st_mtime < newest:
-            subprocess.check_call(["make", "-C", str(HERE), "ref"], stdout=subprocess.DEVNULL)
+            subprocess.check_call(["make", "-C", str(HERE), "ref", f"REFMODS={mods}"], stdout=subprocess.DEVNULL)
 
 
 def _f32(a):
@@ -152,7 +161,7 @@ class WatRef:
 
     def __init__(self):
         if not WATREF_SO.exists():
-            raise FileNotFoundError(f"{WATREF_SO} missing (run `make -C oracle ref` where /root/reference exists)")
+            raise FileNotFoundError(f"{WATREF_SO} missing (build it with WATFFT_REFERENCE set to a wat-fft checkout)")
         self.lib = ctypes.CDLL(str(WATREF_SO))
         self.mem = {}
         for m in self.MODULES:

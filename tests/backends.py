@@ -108,3 +108,59 @@ class GpuBackend:
         out = c.getInputBuffer().reshape(b, n).copy()
         c.dispose()
         return out
+
+
+class StoredWatRef:
+    """Stand-in for oracle.WatRef where the transpiled reference modules are not built: answers with the outputs the
+    reference modules produced for the stored inputs (tests/golden/watref_vectors.npz, tests/golden/make_fixtures.py)
+    and raises LookupError for any other input."""
+
+    SIZES = (4, 8, 16, 32, 64, 128, 256, 1024, 4096)
+
+    def __init__(self):
+        from pathlib import Path
+        self.fix = np.load(Path(__file__).resolve().parent / "golden" / "watref_vectors.npz")
+
+    def signals(self, n):
+        """The stored inputs at size n: re, im (f32 split), il (f32 interleaved), d (f64 interleaved), xr (f64 real)."""
+        import oracle as om
+        if n not in self.SIZES:
+            raise LookupError(f"no stored reference outputs at N={n}")
+        re, im = self.fix[f"in_re_{n}"], self.fix[f"in_im_{n}"]
+        il = np.empty(2 * n, np.float32)
+        il[0::2], il[1::2] = re, im
+        d = np.empty(2 * n)
+        d[0::2], d[1::2] = om.lcg_signal(n, 12345 + n), om.lcg_signal(n, 54321 + n)
+        return {"re": re, "im": im, "il": il, "d": d, "xr": self.fix[f"in_real_{n}"]}
+
+    def _get(self, x, stored, key):
+        if not np.array_equal(np.asarray(x), stored) or key not in self.fix:
+            raise LookupError(f"{key}: input is not a stored one")
+        return self.fix[key].copy()
+
+    def fft_split_f32(self, re, im, inverse=False):
+        n, tag = len(re), "inv" if inverse else "fwd"
+        s = self.signals(n)
+        self._get(im, s["im"], f"split_{tag}_im_{n}")
+        return self._get(re, s["re"], f"split_{tag}_re_{n}"), self.fix[f"split_{tag}_im_{n}"].copy()
+
+    def fft_interleaved_f32(self, data, inverse=False):
+        n = len(data) // 2
+        return self._get(data, self.signals(n)["il"], f"dual_{'inv' if inverse else 'fwd'}_{n}")
+
+    def fft_f64(self, data, inverse=False):
+        n = len(data) // 2
+        return self._get(data, self.signals(n)["d"], f"f64_{'inv' if inverse else 'fwd'}_{n}")
+
+    def rfft_split_f32(self, x):
+        n = len(x)
+        return self._get(x, self.signals(n)["xr"].astype(np.float32), f"rfft32_{n}")
+
+    def irfft_split_f32(self, spec):
+        n = len(spec) - 2
+        self.signals(n)
+        return self._get(spec, self.fix.get(f"rfft32_{n}"), f"irfft32_{n}")
+
+    def rfft_f64(self, x):
+        n = len(x)
+        return self._get(x, self.signals(n)["xr"], f"rfft64_{n}")

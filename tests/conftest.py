@@ -27,8 +27,18 @@ def watref():
     import oracle as om
     om.build()
     if not om.WatRef.available():
-        pytest.skip("oracle/_ref/libwatref.so not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libwatref.so not built (needs WATFFT_REFERENCE, a wat-fft checkout, at build time)")
     return om.WatRef()
+
+
+@pytest.fixture(scope="session")
+def reference():
+    """The reference modules: transpiled (oracle/_ref/libwatref.so) when built, otherwise the outputs stored from them,
+    which answer for the stored inputs only (backends.StoredWatRef)."""
+    import oracle as om
+    from backends import StoredWatRef
+    om.build()
+    return om.WatRef() if om.WatRef.available() else StoredWatRef()
 
 
 @pytest.fixture(scope="session")

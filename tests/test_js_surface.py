@@ -3,6 +3,7 @@ index.js exports every factory the reference's index.js exports, its contexts ca
 exports are synchronous, index.d.ts declares every name the reference's declares, and the N-API shim type-checks against the
 Node-API signatures of the calls it makes (tests/napi_stub/node_api.h).  The behaviour of this surface is tested through its
 Python twin (wat-fft_b200/contexts.py -- same design, same C ABI) in the GPU tests."""
+import os
 import re
 import subprocess
 from pathlib import Path
@@ -12,9 +13,9 @@ import pytest
 ROOT = Path(__file__).resolve().parent.parent
 JS = (ROOT / "wat-fft_b200" / "js" / "index.js").read_text()
 DTS = (ROOT / "wat-fft_b200" / "js" / "index.d.ts").read_text()
-REF = Path("/root/reference")
+REF = Path(os.environ["WATFFT_REFERENCE"]) if os.environ.get("WATFFT_REFERENCE") else None   # a wat-fft checkout
 
-# the reference's public surface (index.js:28-178, index.d.ts:6-250), restated so the test also runs where /root/reference is absent
+# the reference's public surface (index.js:28-178, index.d.ts:6-250), restated so the test also runs without a reference checkout
 REF_FACTORIES = ["createFFTInstance", "createFFTf32Instance", "createRFFTInstance", "createRFFTf32Instance",
                  "createFFT", "createFFTf32", "createRFFT", "createRFFTf32"]
 REF_TYPES = ["FFTExports", "FFTf32Exports", "RFFTExports", "RFFTf32Exports", "FFT", "FFTf32", "RFFT", "RFFTf32"]
@@ -22,8 +23,8 @@ REF_CONTEXT_FIELDS = ["size", "exports", "getInputBuffer", "getOutputBuffer", "f
 
 
 def test_restated_surface_matches_the_reference():
-    if not REF.exists():
-        pytest.skip("reference checkout absent")
+    if REF is None:
+        pytest.skip("reference checkout absent (set WATFFT_REFERENCE)")
     ref_js = (REF / "index.js").read_text()
     assert sorted(re.findall(r"export async function (\w+)", ref_js)) == sorted(REF_FACTORIES)
     ref_dts = (REF / "index.d.ts").read_text()

@@ -15,10 +15,22 @@ ALL = [4, 8, 16, 32, 64, 128, 256, 512, 1024, 2048, 4096, 8192]
 
 
 @pytest.mark.parametrize("n", ALL)
-def test_oracle_bit_exact_vs_reference_modules(oracle, watref, n):
-    rng = np.random.default_rng(n)
-    re = rng.uniform(-1, 1, n).astype(np.float32)
-    im = rng.uniform(-1, 1, n).astype(np.float32)
+def test_oracle_bit_exact_vs_reference_modules(oracle, reference, n):
+    """Random inputs through the transpiled modules when they are built; otherwise the inputs stored with the modules'
+    outputs (tests/golden), which exist for FIX_SIZES."""
+    watref = reference
+    if isinstance(reference, om.WatRef):
+        rng = np.random.default_rng(n)
+        re = rng.uniform(-1, 1, n).astype(np.float32)
+        im = rng.uniform(-1, 1, n).astype(np.float32)
+        ds = [rng.uniform(-1, 1, 2 * n) for _ in range(2)]
+        x32 = rng.uniform(-1, 1, n).astype(np.float32) if n >= 32 else None
+        x64 = rng.uniform(-1, 1, n) if n >= 8 else None
+    else:
+        if n not in FIX_SIZES:
+            pytest.skip(f"no stored reference outputs at N={n} (needs WATFFT_REFERENCE, a wat-fft checkout)")
+        s = reference.signals(n)
+        re, im, ds, x32, x64 = s["re"], s["im"], [s["d"], s["d"]], s["xr"].astype(np.float32), s["xr"]
     for inv in (False, True):
         a, b = oracle.fft_split_f32(re, im, inv), watref.fft_split_f32(re, im, inv)
         assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]), ("split", n, inv)
@@ -29,19 +41,19 @@ def test_oracle_bit_exact_vs_reference_modules(oracle, watref, n):
             assert np.max(np.abs(a - b)) <= 4e-7 * np.linalg.norm(x)
         else:
             assert np.array_equal(a, b), ("dual", n, inv)
-        d = rng.uniform(-1, 1, 2 * n)
+        d = ds[inv]
         a, b = oracle.fft_f64(d, inv), watref.fft_f64(d, inv)
         if n == 16:             # $fft_16 codelet (fft_combined.wat:175-356)
             assert np.max(np.abs(a - b)) <= 4e-16 * np.linalg.norm(d)
         else:
             assert np.array_equal(a, b), ("f64", n, inv)
     if n >= 32:
-        x = rng.uniform(-1, 1, n).astype(np.float32)
+        x = x32
         s = watref.rfft_split_f32(x)
         assert np.array_equal(oracle.rfft_split_f32(x), s), ("rfft32", n)
         assert np.array_equal(oracle.irfft_split_f32(s), watref.irfft_split_f32(s)), ("irfft32", n)
     if n >= 8:
-        x = rng.uniform(-1, 1, n)
+        x = x64
         a, b = oracle.rfft_f64(x), watref.rfft_f64(x)
         if n in (8, 32):        # $rfft_8 / $rfft_32 fused codelets
             assert np.max(np.abs(a - b)) <= 8e-16 * np.linalg.norm(x)
