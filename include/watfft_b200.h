@@ -214,6 +214,21 @@ WFB_API int wfb_stft_exec(wfb_stft *st, int flags);     /* flags as wfb_exec */
 WFB_API int wfb_stft_exec_device(wfb_stft *st, const float *d_samples, void *d_out, void *stream);
 /* Algorithmic bytes of one exec: every sample read once + the output written once. */
 WFB_API size_t wfb_stft_algorithmic_bytes(wfb_stft *st);
+/* Inverse of a WFB_STFT_COMPLEX spectrogram (an extension: the reference has no inverse).  Weighted overlap-add, the
+ * least-squares estimate (what torch.istft(..., center=False) computes):
+ *   y_f = the c2r of row f (1/N normalised, real parts of DC and Nyquist only), its first `window` samples used;
+ *   num[t] = sum_f w[t-f*hop] y_f[t-f*hop],  D[t] = sum_f w[t-f*hop]^2  over the frames with 0 <= t-f*hop < window;
+ *   x[t] = num[t] / D[t] where D[t] >= 1e-11, else 0  (window edges that are 0, gaps when hop > window), and 0 on
+ *   [(frames-1)*hop + window, num_samples).
+ * Unmodified spectra give back the signal wherever D >= 1e-11, to f32 rounding.  Every sum runs in increasing f, so the
+ * result is bitwise repeatable.  WFB_ERR_UNSUPPORTED for a WFB_STFT_DB handle (magnitudes in dB cannot be inverted).
+ * The inverse's twiddle tables are built by the first inverse call, not at creation.
+ * wfb_stft_exec_inverse runs over the handle's own buffers: H2D of wfb_stft_host_output, kernel, D2H of
+ * wfb_stft_host_samples, sync (flags as wfb_exec).  wfb_stft_exec_inverse_device reads frames x bins complex values at
+ * d_spectra (8-byte aligned) and writes num_samples floats at d_samples (any float address); the two must not overlap.
+ * The stream contract is wfb_exec_device's. */
+WFB_API int wfb_stft_exec_inverse(wfb_stft *st, int flags);
+WFB_API int wfb_stft_exec_inverse_device(wfb_stft *st, const void *d_spectra, float *d_samples, void *stream);
 
 #ifdef __cplusplus
 }

@@ -78,6 +78,8 @@ SYMBOLS = {
     "wfb_stft_exec": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
     "wfb_stft_exec_device": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
     "wfb_stft_algorithmic_bytes": (ctypes.c_size_t, [ctypes.c_void_p]),
+    "wfb_stft_exec_inverse": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
+    "wfb_stft_exec_inverse_device": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
 }
 WINDOWS = {"hann": 0, "hamming": 1, "blackman": 2, "blackmanHarris": 3, "rectangular": 4}
 STFT_DB, STFT_COMPLEX = 0, 1

@@ -1072,6 +1072,10 @@ struct wfb_stft {
     size_t out_bytes;
     float db_floor, inv_range;
     cudaStream_t stream;
+    // inverse (wfb_stft_exec_inverse*): built on the first inverse call, so a forward-only handle never pays for it
+    const IstftVariant *inv_variant;
+    void *d_tw_inv;                    // conjugated stage tables of the inverse kernel's core plan
+    cudaEvent_t inv_ready;             // recorded behind their upload: later calls on other streams wait for it
 };
 
 // WINDOW_FUNCTIONS of playground/src/spectrogram.js:1-25, evaluated in double like the JS, stored as f32
@@ -1152,6 +1156,7 @@ wfb_stft *wfb_stft_create(int fft_size, int zero_padding, int hop, int window_ty
     st->out_bytes = (size_t)st->frames * (fft_size / 2 + 1) * sizeof(float) * (mode == WFB_STFT_COMPLEX ? 2 : 1);
     for (const StftVariant &v : variants_stft()) if (v.core_n == fft_size / 2) st->variant = &v;
     if (!st->variant) { *err = WFB_ERR_BAD_SIZE; delete st; return nullptr; }
+    for (const IstftVariant &v : variants_istft()) if (v.core_n == fft_size / 2) st->inv_variant = &v;
     *err = stft_init(st);
     if (*err) { wfb_stft_destroy(st); return nullptr; }
     return st;
@@ -1161,8 +1166,9 @@ void wfb_stft_destroy(wfb_stft *st) {
     if (!st) return;
     cudaSetDevice(st->device);
     if (st->stream) { cudaStreamSynchronize(st->stream); cudaStreamDestroy(st->stream); }
-    void *d[] = {st->d_tw, st->d_tw_span, st->d_rtw, st->d_window, st->d_samples, st->d_out};
+    void *d[] = {st->d_tw, st->d_tw_span, st->d_rtw, st->d_window, st->d_samples, st->d_out, st->d_tw_inv};
     for (void *p : d) if (p) cudaFree(p);
+    if (st->inv_ready) cudaEventDestroy(st->inv_ready);
     if (st->h_samples) cudaFreeHost(st->h_samples);
     if (st->h_out) cudaFreeHost(st->h_out);
     delete st;
@@ -1216,6 +1222,72 @@ int wfb_stft_exec(wfb_stft *st, int flags) {
     int rc = wfb_stft_exec_device(st, (const float *)st->d_samples, st->d_out, nullptr);
     if (rc) return rc;
     if (flags & WFB_STAGE_D2H) CK(cudaMemcpyAsync(st->h_out, st->d_out, st->out_bytes, cudaMemcpyDeviceToHost, st->stream));
+    if (flags & WFB_SYNC) CK(cudaStreamSynchronize(st->stream));
+    return WFB_OK;
+}
+
+// Inverse stage tables of the inverse kernel's core plan (the c2r convention: the forward base table conjugated, no
+// W_8 opening constants), uploaded on `cs` ahead of the launch that follows; calls on any other stream wait for the upload.
+static int stft_inverse_tables(wfb_stft *st, cudaStream_t cs) {
+    if (st->d_tw_inv) {
+        CK(cudaStreamWaitEvent(cs, st->inv_ready, 0));
+        return WFB_OK;
+    }
+    const int m = st->fft_size / 2;
+    std::vector<float> bre, bim, inv;
+    base_twiddles<float>(m >= WFB_DERIVE_MIN_N ? TW_EXACT : TW_F32_SPLIT, m, m, bre, bim);
+    stage_tables<float>(st->inv_variant->radices, m, bre, bim, true, inv);
+    if (inv.empty()) inv.assign(2, 0.0f);
+    void *d = nullptr;
+    CK(cudaMalloc(&d, inv.size() * sizeof(float)));
+    cudaError_t e = cudaMemcpyAsync(d, inv.data(), inv.size() * sizeof(float), cudaMemcpyHostToDevice, cs);
+    if (e == cudaSuccess && !st->inv_ready) e = cudaEventCreateWithFlags(&st->inv_ready, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaEventRecord(st->inv_ready, cs);
+    if (e != cudaSuccess) { cudaFree(d); return cuda_fail(e, "stft inverse tables"); }
+    st->d_tw_inv = d;
+    return WFB_OK;
+}
+
+int wfb_stft_exec_inverse_device(wfb_stft *st, const void *d_spectra, float *d_samples, void *stream) {
+    if (!st || !d_spectra || !d_samples) return WFB_ERR_BAD_ARG;
+    if ((st->mode & 0xFF) != WFB_STFT_COMPLEX) return WFB_ERR_UNSUPPORTED;      // dB magnitudes have no inverse
+    if (((uintptr_t)d_spectra % 8) != 0) return WFB_ERR_BAD_ARG;
+    const uintptr_t s0 = (uintptr_t)d_spectra, s1 = s0 + st->out_bytes;
+    const uintptr_t x0 = (uintptr_t)d_samples, x1 = x0 + (size_t)st->num_samples * sizeof(float);
+    if (s0 < x1 && x0 < s1) return WFB_ERR_BAD_ARG;
+    if (!st->inv_variant) return WFB_ERR_BAD_SIZE;
+    CK(cudaSetDevice(st->device));
+    cudaStream_t cs = stream ? (cudaStream_t)stream : st->stream;
+    int rc = stft_inverse_tables(st, cs);
+    if (rc) return rc;
+    const IstftVariant &v = *st->inv_variant;
+    const int X = v.frames_per_round;
+    // a CTA owns P hops of output and recomputes the halo = ceil(W/H) - 1 frames before them: P + halo is a whole number
+    // of rounds and P >= 10 halo (<= 10 % recomputed frames), and at least 16 frames
+    const long H = st->hop, W = st->wsize, halo = (W + H - 1) / H - 1;
+    const long rounds = std::max((11 * halo + X - 1) / X, (16L + X - 1) / X);
+    IstftParams ip;
+    ip.spectra = (const float2 *)d_spectra; ip.out = d_samples; ip.window = (const float *)st->d_window;
+    ip.tw = st->d_tw_inv; ip.rtw = st->d_rtw;
+    ip.frames = st->frames; ip.num_samples = st->num_samples;
+    ip.tile_frames = rounds * X - halo;
+    ip.hop = st->hop; ip.wsize = st->wsize; ip.halo = (int)halo;
+    ip.inv_hop = 1.0f / (float)st->hop;
+    const long tiles = (st->num_samples + ip.tile_frames * H - 1) / (ip.tile_frames * H);
+    cudaError_t e = v.launch(ip, tiles, cs);
+    if (e != cudaSuccess) return cuda_fail(e, "stft inverse launch");
+    return WFB_OK;
+}
+
+int wfb_stft_exec_inverse(wfb_stft *st, int flags) {
+    if (!st || !st->d_samples) return WFB_ERR_BAD_ARG;
+    if ((st->mode & 0xFF) != WFB_STFT_COMPLEX) return WFB_ERR_UNSUPPORTED;
+    if ((flags & (WFB_STAGE_H2D | WFB_STAGE_D2H)) && !st->h_out) return WFB_ERR_NO_HOST_BUFFERS;
+    CK(cudaSetDevice(st->device));
+    if (flags & WFB_STAGE_H2D) CK(cudaMemcpyAsync(st->d_out, st->h_out, st->out_bytes, cudaMemcpyHostToDevice, st->stream));
+    int rc = wfb_stft_exec_inverse_device(st, st->d_out, (float *)st->d_samples, nullptr);
+    if (rc) return rc;
+    if (flags & WFB_STAGE_D2H) CK(cudaMemcpyAsync(st->h_samples, st->d_samples, st->num_samples * sizeof(float), cudaMemcpyDeviceToHost, st->stream));
     if (flags & WFB_SYNC) CK(cudaStreamSynchronize(st->stream));
     return WFB_OK;
 }

@@ -2575,4 +2575,138 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_span(const __grid_const
     claim_epilogue(sp.ctr);
 }
 
+// ----------------------------------------------------------------------------------------
+// Inverse STFT (extension, no reference counterpart): the weighted overlap-add / least-squares estimate of a signal from
+// the complex spectra the STFT_MODE_COMPLEX kernels write,
+//   y_f = c2r(X_f) (1/N, real parts of DC and Nyquist),   x[t] = sum_f w[t-fH] y_f[t-fH] / sum_f w[t-fH]^2
+// (0 where the denominator is below 1e-11, i.e. where no frame carries weight), in ONE kernel: c2r pre-process, inverse
+// core, window multiply and overlap-add fused, every spectrum read once and every sample written once.
+//   * A CTA owns the output samples of `tile_frames` hops, [a, b), and nothing else writes them.  It recomputes the
+//     ceil(W/H) - 1 earlier frames that reach into [a, b) (the halo) instead of exchanging seams with its neighbours.
+//   * Frames are computed X at a time (a round), one per thread group, and land windowed in shared memory.  One thread
+//     per output sample then adds the round's contributions to what earlier rounds left in a carry buffer (increasing
+//     frame order throughout, so the result does not depend on the tiling) and, for the samples no later frame can
+//     reach, divides by the window-square sum formed from the window in shared memory and stores.
+// Shared memory: [X scratch rows, reused as the windowed frames][2 carry buffers of N floats][window, M float2].
+// ----------------------------------------------------------------------------------------
+struct IstftParams {
+    const float2 *spectra;     // [frames][M+1] complex bins
+    float *out;                // [num_samples]
+    const float *window;       // [wsize] window function values (f32), host-built
+    const void *tw, *rtw;      // inverse stage tables / W_N^k of the c2r core
+    long frames, num_samples;
+    long tile_frames;          // hops of output one CTA owns
+    int hop, wsize, halo;      // halo = ceil(wsize / hop) - 1
+    float inv_hop;             // 1 / hop (for small quotients, corrected exactly)
+};
+
+template <class PL, int PADQ, int X> __host__ __device__ constexpr size_t istft_smem_bytes() {
+    return sizeof(float) * 2 * (size_t)padded_size<PADQ>(PL::N) * X + sizeof(float) * 4 * (size_t)PL::N + sizeof(float2) * (size_t)PL::N;
+}
+
+template <class PL, int X, int PADQ, int MINB>
+__global__ void __launch_bounds__(PL::T *X, MINB) k_istft(const __grid_constant__ IstftParams ip) {
+    static_assert(PL::valid(), "plan does not factor N");
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    using R = float;
+    constexpr int M = PL::N, T = PL::T, E = PL::E, HALF = M / 2, PER = (HALF + T - 1) / T, NT = T * X;
+    constexpr int LAST = PL::npass() - 1;
+    constexpr int SROW = 2 * padded_size<PADQ>(M);                      // floats per group row (scratch, then frame)
+    float *work = reinterpret_cast<float *>(smem_raw);
+    float *carry = work + (size_t)X * SROW;                              // two buffers of 2M >= wsize floats
+    float2 *winsm = reinterpret_cast<float2 *>(carry + 4 * M);
+    const float *winf = reinterpret_cast<const float *>(winsm);
+    const int xi = threadIdx.x / T, tid = threadIdx.x % T;
+    const float2 *tw = reinterpret_cast<const float2 *>(ip.tw);
+    const float2 *rtw = reinterpret_cast<const float2 *>(ip.rtw);
+    const int H = ip.hop, W = ip.wsize;
+    {
+        const float2 *w2 = reinterpret_cast<const float2 *>(ip.window);
+        for (int p = threadIdx.x; p < M; p += NT) winsm[p] = 2 * p < W ? __ldg(w2 + p) : make_float2(0.0f, 0.0f);
+    }
+    const long k0 = (long)blockIdx.x * ip.tile_frames;                   // first frame this CTA owns
+    const long a = k0 * H, b = min(a + ip.tile_frames * H, ip.num_samples);
+    // sample offset u (from the round's first frame start) = q*H + r, stepped by NT without dividing
+    const int tq = threadIdx.x / H, tr = threadIdx.x % H, sq = NT / H, sr = NT % H;
+    const long ucov = max((long)(X - 1) * H + W, (long)X * H);          // reach of a round's frames (or its hops)
+    const R sc = 0.5f / (float)M;
+    int cur = 0;
+    __syncthreads();
+    for (long g = max(0L, k0 - ip.halo); g * H < b; g += X) {
+        if (g < ip.frames) {                                             // (CTA-uniform) the round has frames
+            const long f = g + xi;
+            cx<R> *sm = reinterpret_cast<cx<R> *>(work + (size_t)xi * SROW);
+            if (f < ip.frames && f * H < b) {
+                // Hermitian pre-process of k_c2r (scale 0.5/M folded in, real parts only at DC and Nyquist)
+                const float2 *in = ip.spectra + f * (M + 1);
+                static_for<PER>([&](auto I_) {
+                    CIDX(i, I_);
+                    const int k = tid + i * T;
+                    if (k < HALF) {
+                        if (i == 0 && k == 0) {
+                            const float2 a0 = __ldg(in), am = __ldg(in + M);
+                            sm[0] = mk<R>((a0.x + am.x) * sc, (a0.x - am.x) * sc);
+                        }
+                        const int kk = (k == 0) ? HALF : k;
+                        const float2 va = __ldg(in + kk), vb = __ldg(in + (M - kk));
+                        const twd<R> w = ld_tw(rtw + kk);
+                        const R gr = va.x + vb.x, gi = va.y - vb.y, ur = va.x - vb.x, ui = va.y + vb.y;
+                        const R hr = fmaf(w.y, ui, w.x * ur), hi = fmaf(w.ny, ur, w.x * ui);
+                        sm[pad_idx<PADQ>(kk)] = mk<R>(sc * (gr - hi), sc * (gi + hr));
+                        sm[pad_idx<PADQ>(M - kk)] = mk<R>(sc * (gr + hi), sc * (hr - gi));
+                    }
+                });
+            }
+            sync_transform<T, X>(xi);
+            cx<R> x[E];
+            {
+                const cx<R> *base = sm + pad_idx<PADQ>(tid);
+                static_for<E>([&](auto E_) { CIDX(e, E_); x[e] = base[pad_off<PADQ>(e * T)]; });
+            }
+            run_all<R, PL, PADQ, X, true>(x, tw, GTw<R>{nullptr, tw}, sm, tid, xi, true);
+            sync_transform<T, X>(xi);                                    // the group's last reads of its scratch are done
+            float2 *frame = reinterpret_cast<float2 *>(sm);              // y[2p], y[2p+1] times the window (0 past it)
+            static_for<E>([&](auto S_) {
+                CIDX(slot, S_);
+                const int p = tid + out_elem<PL, LAST>(slot) * T;
+                const float2 w = winsm[p];
+                frame[p] = make_float2(x[slot].x * w.x, x[slot].y * w.y);
+            });
+        }
+        __syncthreads();
+        // overlap-add: this round's frames g .. g + flast reach [gH, gH + ucov); samples below (g + X) H are final
+        const long gH = g * H;
+        const int flast = (int)max(-1L, min((long)X - 1, ip.frames - 1 - g));
+        const float *cin = carry + cur * 2 * M;
+        float *cout = carry + (cur ^ 1) * 2 * M;
+        const bool carried = g > max(0L, k0 - ip.halo);                  // an earlier round of this CTA left sums
+        const long u0 = gH < a ? a - gH : 0, uend = min(ucov, b - gH);
+        int q = (int)((gH < a ? k0 - g : 0) + tq), r = tr;              // u0 is a multiple of H
+        for (long u = u0 + threadIdx.x; u < uend; u += NT) {
+            float num = (carried && u < W - H) ? cin[u] : 0.0f;
+            int dmax = -1;                                               // frames q - d with d*H + r < W cover u
+            if (r < W) {
+                const int span = W - 1 - r;
+                dmax = __float2int_rz((float)span * ip.inv_hop);
+                if (dmax * H > span) dmax--;
+                else if ((dmax + 1) * H <= span) dmax++;
+            }
+            for (int d = min(dmax, q); d >= max(0, q - flast); d--) num += work[(q - d) * SROW + d * H + r];
+            if (q < X) {
+                const long fg = g + q;                                   // frames fg - d, every one that exists
+                float den = 0.0f;
+                const int dlo = (int)min(max(0L, fg - (ip.frames - 1)), (long)dmax + 1);
+                for (int d = (int)min((long)dmax, fg); d >= dlo; d--) { const float w = winf[d * H + r]; den = fmaf(w, w, den); }
+                st_stream(ip.out + gH + u, den >= 1e-11f ? num / den : 0.0f);
+            } else {
+                cout[u - (long)X * H] = num;
+            }
+            r += sr; q += sq;
+            if (r >= H) { r -= H; q++; }
+        }
+        cur ^= 1;
+        __syncthreads();
+    }
+}
+
 }  // namespace wfb

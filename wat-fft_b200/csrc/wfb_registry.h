@@ -265,6 +265,21 @@ template <class PL, int X, int MINB, class SPL, int XS, int SMINB, int SPQ, bool
     }
 };
 
+// fused inverse STFT (c2r + window + overlap-add, k_istft): one per FFT size, on the core plan of that size's STFT span
+// kernel (the direct kernel's where there is none); X frames per round
+typedef cudaError_t (*istft_launch_fn)(const IstftParams &ip, long tiles, cudaStream_t s);
+struct IstftVariant {
+    const char *name; int core_n; std::vector<int> radices; istft_launch_fn launch; int frames_per_round;
+};
+const std::vector<IstftVariant> &variants_istft();
+template <class PL, int X, int PQ, int MINB> struct IstftLaunchers {
+    static constexpr size_t smem = istft_smem_bytes<PL, PQ, X>();
+    static cudaError_t launch(const IstftParams &ip, long tiles, cudaStream_t s) {
+        return launch_grid_raw((const void *)k_istft<PL, X, PQ, MINB>, smem, PL::T * X, tiles, (void *)&ip, s);
+    }
+    static IstftVariant make(const char *name) { return IstftVariant{name, PL::N, plan_radices<PL>(), &launch, X}; }
+};
+
 #define XROWS(T) ((T) >= 256 ? 1 : 256 / (T))
 
 // f32 core plans: the reference's split-core stage structure (radix-4, leading radix-2 for odd log2)

@@ -4,7 +4,10 @@ Mirror of `generateSpectrogram({samples, sampleRate, fftContext, hopSize, window
 gain, range})` in playground/src/spectrogram.js:270-372: same arguments (the FFT context is
 replaced by `fftSize`), same returned fields, same numerics to f32 tolerance -- but the per-frame
 JavaScript loop (slice, window, zero-pad, copy, run, magnitude, dB) is a single kernel over all
-frames (csrc/wfb_kernels.cuh k_stft)."""
+frames (csrc/wfb_kernels.cuh k_stft).
+
+The inverse (Spectrogram.inverse, inverseSpectrogram) is an extension with no reference counterpart: the weighted
+overlap-add of the frames' c2r outputs, fused into one kernel as well (k_istft)."""
 from __future__ import annotations
 
 import ctypes
@@ -50,6 +53,15 @@ class Spectrogram:
         C.check(self._lib.wfb_stft_exec_device(self._p, ctypes.c_void_p(d_samples), ctypes.c_void_p(d_out),
                                                ctypes.c_void_p(stream) if stream else None))
 
+    def inverse(self):
+        """Signal from the complex spectra in getOutputBuffer() (weighted overlap-add, see inverseSpectrogram), written
+        to getInputBuffer().  mode="complex" only."""
+        C.check(self._lib.wfb_stft_exec_inverse(self._p, C.EXEC_DEFAULT))
+
+    def inverse_device(self, d_spectra, d_samples, stream=None):
+        C.check(self._lib.wfb_stft_exec_inverse_device(self._p, ctypes.c_void_p(d_spectra), ctypes.c_void_p(d_samples),
+                                                       ctypes.c_void_p(stream) if stream else None))
+
     def algorithmic_bytes(self):
         return self._lib.wfb_stft_algorithmic_bytes(self._p)
 
@@ -80,3 +92,24 @@ def generateSpectrogram(samples, sampleRate, fftSize, hopSize, windowType="hann"
            "windowSize": window, "hopSize": hopSize, "sampleRate": sampleRate}
     sp.dispose()
     return out
+
+
+def inverseSpectrogram(spectra, fftSize, hopSize, windowType="hann", zeroPadding=1, device=0):
+    """Signal from complex STFT frames ([frames][fftSize/2+1][2] float32, the layout of Spectrogram(mode="complex")):
+    the least-squares / weighted overlap-add estimate that torch.istft(..., center=False) also computes,
+        x[t] = sum_f w[t-f*hop] y_f[t-f*hop] / sum_f w[t-f*hop]^2   (0 where that sum is below 1e-11),
+    y_f the 1/N-normalised c2r of frame f (real parts of DC and Nyquist).  Returns (frames-1)*hop + window float32
+    samples; spectra left unmodified give back the analysed signal wherever a frame carries weight."""
+    spectra = np.ascontiguousarray(spectra, np.float32)
+    if spectra.ndim != 3 or spectra.shape[1] != fftSize // 2 + 1 or spectra.shape[2] != 2 or spectra.shape[0] < 1:
+        raise ValueError(f"spectra must be [frames][{fftSize // 2 + 1}][2], got {spectra.shape}")
+    window = fftSize // zeroPadding
+    length = (spectra.shape[0] - 1) * hopSize + window
+    sp = Spectrogram(length, fftSize, hopSize, windowType, zeroPadding, mode="complex", device=device)
+    try:
+        assert sp.numFrames == spectra.shape[0]
+        sp.getOutputBuffer()[:] = spectra
+        sp.inverse()
+        return sp.getInputBuffer().copy()
+    finally:
+        sp.dispose()
