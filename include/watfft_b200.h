@@ -197,17 +197,31 @@ WFB_API int wfb_reference_twiddles(int flavour, int n, int count, void *re, void
  *   frames = floor((num_samples - window) / hop) + 1,  window = fft_size / zero_padding,
  *   bins   = fft_size/2 + 1.
  * Output, mode WFB_STFT_DB: float [frames][bins] in [0,1] (bins 0..2 forced to 0, :338-342);
- *         mode WFB_STFT_COMPLEX: float [frames][bins][2] (the raw spectra of the windowed frames). */
+ *         mode WFB_STFT_COMPLEX: float [frames][bins][2] (the raw spectra of the windowed frames).
+ * Batches: wfb_stft_create_ex takes `batch` >= 1 equal-length signals in one handle, one launch for all of them.
+ *   Input float [batch][num_samples], contiguous; output float [batch][frames][bins] (dB) or
+ *   float [batch][frames][bins][2] (complex); `frames` (wfb_stft_frames) stays the count of ONE signal.  Every signal's
+ *   rows are exactly what a single-signal handle computes for it: no frame reads samples of another signal, and the
+ *   dB normalisation uses the fixed gain/range only.  wfb_stft_create is wfb_stft_create_ex with batch = 1.
+ *   wfb_stft_output_bytes, wfb_stft_algorithmic_bytes and the pinned buffers cover the whole batch.  WFB_ERR_BAD_ARG
+ *   for batch < 1 or a batch whose bytes overflow size_t.
+ *   Alignment: the bulk-copy kernels (by default N = 1024, 2048 and 8192) need 16-byte aligned frame starts in every
+ *   signal, the direct kernel's 64-bit loads 8-byte aligned ones.  With batch > 1 they are taken only when num_samples
+ *   is a multiple of 4 (respectively 2) floats; otherwise the same results come from the direct kernel with narrower
+ *   loads, as for an unaligned d_samples. */
 typedef struct wfb_stft wfb_stft;
 enum { WFB_WINDOW_HANN = 0, WFB_WINDOW_HAMMING = 1, WFB_WINDOW_BLACKMAN = 2, WFB_WINDOW_BLACKMAN_HARRIS = 3,
        WFB_WINDOW_RECTANGULAR = 4 };
 enum { WFB_STFT_DB = 0, WFB_STFT_COMPLEX = 1 };
 WFB_API wfb_stft *wfb_stft_create(int fft_size, int zero_padding, int hop, int window_type, long num_samples,
                                   int mode, float gain_db, float range_db, int device, int flags, int *err);
+WFB_API wfb_stft *wfb_stft_create_ex(int fft_size, int zero_padding, int hop, int window_type, long num_samples,
+                                     long batch, int mode, float gain_db, float range_db, int device, int flags, int *err);
 WFB_API void wfb_stft_destroy(wfb_stft *st);
-WFB_API long wfb_stft_frames(wfb_stft *st);
+WFB_API long wfb_stft_frames(wfb_stft *st);             /* per signal */
+WFB_API long wfb_stft_batch(wfb_stft *st);
 WFB_API int wfb_stft_bins(wfb_stft *st);
-WFB_API void *wfb_stft_host_samples(wfb_stft *st);      /* pinned, num_samples floats */
+WFB_API void *wfb_stft_host_samples(wfb_stft *st);      /* pinned, batch x num_samples floats */
 WFB_API void *wfb_stft_host_output(wfb_stft *st);       /* pinned, wfb_stft_output_bytes() */
 WFB_API size_t wfb_stft_output_bytes(wfb_stft *st);
 WFB_API int wfb_stft_exec(wfb_stft *st, int flags);     /* flags as wfb_exec */
@@ -224,9 +238,10 @@ WFB_API size_t wfb_stft_algorithmic_bytes(wfb_stft *st);
  * result is bitwise repeatable.  WFB_ERR_UNSUPPORTED for a WFB_STFT_DB handle (magnitudes in dB cannot be inverted).
  * The inverse's twiddle tables are built by the first inverse call, not at creation.
  * wfb_stft_exec_inverse runs over the handle's own buffers: H2D of wfb_stft_host_output, kernel, D2H of
- * wfb_stft_host_samples, sync (flags as wfb_exec).  wfb_stft_exec_inverse_device reads frames x bins complex values at
- * d_spectra (8-byte aligned) and writes num_samples floats at d_samples (any float address); the two must not overlap.
- * The stream contract is wfb_exec_device's. */
+ * wfb_stft_host_samples, sync (flags as wfb_exec).  wfb_stft_exec_inverse_device reads batch x frames x bins complex
+ * values at d_spectra (8-byte aligned) and writes batch x num_samples floats at d_samples (any float address); the two
+ * must not overlap.  Each signal of a batch is reconstructed from its own frames only, exactly as by a single-signal
+ * handle.  The stream contract is wfb_exec_device's. */
 WFB_API int wfb_stft_exec_inverse(wfb_stft *st, int flags);
 WFB_API int wfb_stft_exec_inverse_device(wfb_stft *st, const void *d_spectra, float *d_samples, void *stream);
 

@@ -69,8 +69,11 @@ SYMBOLS = {
     "wfb_reference_twiddles": (ctypes.c_int, [ctypes.c_int] * 3 + [ctypes.c_void_p] * 2),
     "wfb_stft_create": (ctypes.c_void_p, [ctypes.c_int] * 4 + [ctypes.c_long, ctypes.c_int, ctypes.c_float, ctypes.c_float,
                                            ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_int)]),
+    "wfb_stft_create_ex": (ctypes.c_void_p, [ctypes.c_int] * 4 + [ctypes.c_long, ctypes.c_long, ctypes.c_int, ctypes.c_float,
+                                              ctypes.c_float, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_int)]),
     "wfb_stft_destroy": (None, [ctypes.c_void_p]),
     "wfb_stft_frames": (ctypes.c_long, [ctypes.c_void_p]),
+    "wfb_stft_batch": (ctypes.c_long, [ctypes.c_void_p]),
     "wfb_stft_bins": (ctypes.c_int, [ctypes.c_void_p]),
     "wfb_stft_host_samples": (ctypes.c_void_p, [ctypes.c_void_p]),
     "wfb_stft_host_output": (ctypes.c_void_p, [ctypes.c_void_p]),

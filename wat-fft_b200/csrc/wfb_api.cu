@@ -1065,11 +1065,11 @@ int wfb_pcie_probe(int device, size_t bytes, int iters, double gbs[4]) {
 // ----------------------------------------------------------------------------------------
 struct wfb_stft {
     int fft_size, wsize, hop, mode, device, flags;
-    long num_samples, frames;
+    long num_samples, frames, batch;   // frames per signal; batch signals of num_samples each
     const StftVariant *variant;
     void *d_tw, *d_tw_span, *d_rtw, *d_window, *d_samples, *d_out;
     void *h_samples, *h_out;
-    size_t out_bytes;
+    size_t in_bytes, out_bytes;        // whole batch
     float db_floor, inv_range;
     cudaStream_t stream;
     // inverse (wfb_stft_exec_inverse*): built on the first inverse call, so a forward-only handle never pays for it
@@ -1120,13 +1120,13 @@ static int stft_init(wfb_stft *st) {
     if (!fwd_span.empty() && (rc = up(&st->d_tw_span, fwd_span))) return rc;
     CK(cudaDeviceSynchronize());      // the uploads above ran on the legacy stream; the plan's stream does not order against it
     if (!(st->flags & WFB_PLAN_NO_DEVICE_BUFFERS)) {
-        if (cudaMalloc(&st->d_samples, st->num_samples * sizeof(float)) != cudaSuccess) { cudaGetLastError(); return WFB_ERR_ALLOC; }
+        if (cudaMalloc(&st->d_samples, st->in_bytes) != cudaSuccess) { cudaGetLastError(); return WFB_ERR_ALLOC; }
         if (cudaMalloc(&st->d_out, st->out_bytes) != cudaSuccess) { cudaGetLastError(); return WFB_ERR_ALLOC; }
     }
     if (!(st->flags & WFB_PLAN_NO_HOST_BUFFERS)) {
-        if (cudaHostAlloc(&st->h_samples, st->num_samples * sizeof(float), cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); return WFB_ERR_ALLOC; }
+        if (cudaHostAlloc(&st->h_samples, st->in_bytes, cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); return WFB_ERR_ALLOC; }
         if (cudaHostAlloc(&st->h_out, st->out_bytes, cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); return WFB_ERR_ALLOC; }
-        memset(st->h_samples, 0, st->num_samples * sizeof(float));
+        memset(st->h_samples, 0, st->in_bytes);
         memset(st->h_out, 0, st->out_bytes);
     }
     return WFB_OK;
@@ -1136,6 +1136,11 @@ extern "C" {
 
 wfb_stft *wfb_stft_create(int fft_size, int zero_padding, int hop, int window_type, long num_samples, int mode,
                           float gain_db, float range_db, int device, int flags, int *err) {
+    return wfb_stft_create_ex(fft_size, zero_padding, hop, window_type, num_samples, 1, mode, gain_db, range_db, device, flags, err);
+}
+
+wfb_stft *wfb_stft_create_ex(int fft_size, int zero_padding, int hop, int window_type, long num_samples, long batch, int mode,
+                             float gain_db, float range_db, int device, int flags, int *err) {
     int dummy;
     if (!err) err = &dummy;
     if (!is_pow2(fft_size) || fft_size < 64 || fft_size > 8192) { *err = WFB_ERR_BAD_SIZE; return nullptr; }
@@ -1144,16 +1149,25 @@ wfb_stft *wfb_stft_create(int fft_size, int zero_padding, int hop, int window_ty
         !(range_db > 0.0f)) { *err = WFB_ERR_BAD_ARG; return nullptr; }
     const int wsize = fft_size / zero_padding;
     if (num_samples < wsize) { *err = WFB_ERR_BAD_ARG; return nullptr; }      // "Audio too short" (spectrogram.js:299-301)
+    // the whole batch's input and output must be addressable: batch * num_samples floats, batch * frames * bins values
+    const size_t frames = (size_t)((num_samples - wsize) / hop + 1);
+    const size_t row_bytes = (size_t)(fft_size / 2 + 1) * sizeof(float) * (mode == WFB_STFT_COMPLEX ? 2 : 1);
+    size_t in_bytes, out_bytes;
+    if (batch < 1 || __builtin_mul_overflow((size_t)num_samples, sizeof(float), &in_bytes) ||
+        __builtin_mul_overflow(in_bytes, (size_t)batch, &in_bytes) || __builtin_mul_overflow(frames, row_bytes, &out_bytes) ||
+        __builtin_mul_overflow(out_bytes, (size_t)batch, &out_bytes)) { *err = WFB_ERR_BAD_ARG; return nullptr; }
     *err = check_device(device);
     if (*err) return nullptr;
     wfb_stft *st = new wfb_stft();
     st->fft_size = fft_size; st->wsize = wsize; st->hop = hop; st->device = device; st->flags = flags;
     st->mode = mode | (window_type << 8);
     st->num_samples = num_samples;
-    st->frames = (num_samples - wsize) / hop + 1;
+    st->frames = (long)frames;
+    st->batch = batch;
     st->db_floor = gain_db - range_db;
     st->inv_range = 1.0f / range_db;
-    st->out_bytes = (size_t)st->frames * (fft_size / 2 + 1) * sizeof(float) * (mode == WFB_STFT_COMPLEX ? 2 : 1);
+    st->in_bytes = in_bytes;
+    st->out_bytes = out_bytes;
     for (const StftVariant &v : variants_stft()) if (v.core_n == fft_size / 2) st->variant = &v;
     if (!st->variant) { *err = WFB_ERR_BAD_SIZE; delete st; return nullptr; }
     for (const IstftVariant &v : variants_istft()) if (v.core_n == fft_size / 2) st->inv_variant = &v;
@@ -1175,11 +1189,12 @@ void wfb_stft_destroy(wfb_stft *st) {
 }
 
 long wfb_stft_frames(wfb_stft *st) { return st ? st->frames : 0; }
+long wfb_stft_batch(wfb_stft *st) { return st ? st->batch : 0; }
 int wfb_stft_bins(wfb_stft *st) { return st ? st->fft_size / 2 + 1 : 0; }
 void *wfb_stft_host_samples(wfb_stft *st) { return st ? st->h_samples : nullptr; }
 void *wfb_stft_host_output(wfb_stft *st) { return st ? st->h_out : nullptr; }
 size_t wfb_stft_output_bytes(wfb_stft *st) { return st ? st->out_bytes : 0; }
-size_t wfb_stft_algorithmic_bytes(wfb_stft *st) { return st ? (size_t)st->num_samples * sizeof(float) + st->out_bytes : 0; }
+size_t wfb_stft_algorithmic_bytes(wfb_stft *st) { return st ? st->in_bytes + st->out_bytes : 0; }
 
 int wfb_stft_exec_device(wfb_stft *st, const float *d_samples, void *d_out, void *stream) {
     if (!st || !d_samples || !d_out) return WFB_ERR_BAD_ARG;
@@ -1187,24 +1202,27 @@ int wfb_stft_exec_device(wfb_stft *st, const float *d_samples, void *d_out, void
     StftParams sp;
     sp.samples = d_samples; sp.window = (const float *)st->d_window; sp.out = d_out;
     sp.tw = st->d_tw; sp.rtw = st->d_rtw;
-    sp.frames = st->frames; sp.hop = st->hop; sp.wsize = st->wsize; sp.mode = st->mode & 0xFF;
+    sp.frames = st->frames; sp.batch = st->batch; sp.num_samples = st->num_samples; sp.hop = st->hop; sp.wsize = st->wsize; sp.mode = st->mode & 0xFF;
     sp.db_floor = st->db_floor; sp.inv_range = st->inv_range; sp.inv_half_n = 2.0f / (float)st->fft_size;
     sp.ctr = nullptr;
     sp.span_bytes = 0;
-    sp.aligned8 = ((uintptr_t)d_samples % 8) == 0;      // a caller's pointer may be any float address (scalar loads then)
+    sp.tiles = 0; sp.tps = sp.tps_magic = 0; sp.tps_shift = 0;      // (set by the persistent kernels' launchers)
+    // a caller's pointer may be any float address (scalar loads then); the rows of a batch keep the base's alignment only
+    // when num_samples is a multiple of 2 (8 bytes) or 4 (16 bytes, the bulk-copy kernels)
+    sp.aligned8 = ((uintptr_t)d_samples % 8) == 0 && (st->batch == 1 || st->num_samples % 2 == 0);
+    const bool rows16 = ((uintptr_t)d_samples % 16) == 0 && (st->batch == 1 || st->num_samples % 4 == 0);
     // fast dB path: v = lg_a * log2(|2 X|^2) + lg_b  ==  (10 log10(|X|^2 c^2) - floor) / range,  c = 2 / fft_size
     sp.lg_a = 3.0102999566398120f * st->inv_range;
     sp.lg_b = sp.lg_a * (2.0f * log2f(sp.inv_half_n) - 2.0f) - st->db_floor * st->inv_range;
     // frames are TMA-copyable when their starts are 16-byte aligned (hop % 4 == 0, aligned base)
     static const int pipe_min = [] { const char *e = getenv("WFB_STFT_PIPE_MIN_N"); return e ? atoi(e) : 8192; }();
-    const bool pipe = st->fft_size >= pipe_min && st->hop % 4 == 0 && st->wsize % 4 == 0 && ((uintptr_t)d_samples % 16) == 0;
+    const bool pipe = st->fft_size >= pipe_min && st->hop % 4 == 0 && st->wsize % 4 == 0 && rows16;
     cudaStream_t cs = stream ? (cudaStream_t)stream : st->stream;
     // span kernel: whole tiles of overlapping frames as one bulk copy (16-byte aligned frame starts and sizes)
     const char *span_env = getenv("WFB_STFT_SPAN");             // (read per call: tests and A/B runs flip it)
     const bool span_on = span_env ? atoi(span_env) != 0 : st->variant->span_default;      // WFB_STFT_SPAN=1 forces, =0 forbids
     cudaError_t e = cudaErrorInvalidConfiguration;
-    if (span_on && st->variant->launch_span && st->hop % 4 == 0 && st->wsize % 4 == 0 && ((uintptr_t)d_samples % 16) == 0 &&
-        ((uintptr_t)d_out % 16) == 0) {
+    if (span_on && st->variant->launch_span && st->hop % 4 == 0 && st->wsize % 4 == 0 && rows16 && ((uintptr_t)d_out % 16) == 0) {
         StftParams ss = sp;
         if (st->d_tw_span) ss.tw = st->d_tw_span;
         e = st->variant->launch_span(ss, cs);
@@ -1218,7 +1236,7 @@ int wfb_stft_exec(wfb_stft *st, int flags) {
     if (!st || !st->d_samples) return WFB_ERR_BAD_ARG;
     if ((flags & (WFB_STAGE_H2D | WFB_STAGE_D2H)) && !st->h_samples) return WFB_ERR_NO_HOST_BUFFERS;
     CK(cudaSetDevice(st->device));
-    if (flags & WFB_STAGE_H2D) CK(cudaMemcpyAsync(st->d_samples, st->h_samples, st->num_samples * sizeof(float), cudaMemcpyHostToDevice, st->stream));
+    if (flags & WFB_STAGE_H2D) CK(cudaMemcpyAsync(st->d_samples, st->h_samples, st->in_bytes, cudaMemcpyHostToDevice, st->stream));
     int rc = wfb_stft_exec_device(st, (const float *)st->d_samples, st->d_out, nullptr);
     if (rc) return rc;
     if (flags & WFB_STAGE_D2H) CK(cudaMemcpyAsync(st->h_out, st->d_out, st->out_bytes, cudaMemcpyDeviceToHost, st->stream));
@@ -1253,7 +1271,7 @@ int wfb_stft_exec_inverse_device(wfb_stft *st, const void *d_spectra, float *d_s
     if ((st->mode & 0xFF) != WFB_STFT_COMPLEX) return WFB_ERR_UNSUPPORTED;      // dB magnitudes have no inverse
     if (((uintptr_t)d_spectra % 8) != 0) return WFB_ERR_BAD_ARG;
     const uintptr_t s0 = (uintptr_t)d_spectra, s1 = s0 + st->out_bytes;
-    const uintptr_t x0 = (uintptr_t)d_samples, x1 = x0 + (size_t)st->num_samples * sizeof(float);
+    const uintptr_t x0 = (uintptr_t)d_samples, x1 = x0 + st->in_bytes;
     if (s0 < x1 && x0 < s1) return WFB_ERR_BAD_ARG;
     if (!st->inv_variant) return WFB_ERR_BAD_SIZE;
     CK(cudaSetDevice(st->device));
@@ -1271,10 +1289,10 @@ int wfb_stft_exec_inverse_device(wfb_stft *st, const void *d_spectra, float *d_s
     ip.tw = st->d_tw_inv; ip.rtw = st->d_rtw;
     ip.frames = st->frames; ip.num_samples = st->num_samples;
     ip.tile_frames = rounds * X - halo;
+    ip.tiles = (st->num_samples + ip.tile_frames * H - 1) / (ip.tile_frames * H);
     ip.hop = st->hop; ip.wsize = st->wsize; ip.halo = (int)halo;
     ip.inv_hop = 1.0f / (float)st->hop;
-    const long tiles = (st->num_samples + ip.tile_frames * H - 1) / (ip.tile_frames * H);
-    cudaError_t e = v.launch(ip, tiles, cs);
+    cudaError_t e = v.launch(ip, ip.tiles * st->batch, cs);
     if (e != cudaSuccess) return cuda_fail(e, "stft inverse launch");
     return WFB_OK;
 }
@@ -1287,7 +1305,7 @@ int wfb_stft_exec_inverse(wfb_stft *st, int flags) {
     if (flags & WFB_STAGE_H2D) CK(cudaMemcpyAsync(st->d_out, st->h_out, st->out_bytes, cudaMemcpyHostToDevice, st->stream));
     int rc = wfb_stft_exec_inverse_device(st, st->d_out, (float *)st->d_samples, nullptr);
     if (rc) return rc;
-    if (flags & WFB_STAGE_D2H) CK(cudaMemcpyAsync(st->h_samples, st->d_samples, st->num_samples * sizeof(float), cudaMemcpyDeviceToHost, st->stream));
+    if (flags & WFB_STAGE_D2H) CK(cudaMemcpyAsync(st->h_samples, st->d_samples, st->in_bytes, cudaMemcpyDeviceToHost, st->stream));
     if (flags & WFB_SYNC) CK(cudaStreamSynchronize(st->stream));
     return WFB_OK;
 }

@@ -2195,21 +2195,37 @@ __device__ __forceinline__ void park_upper_half(const cx<R> (&x)[PL::E], cx<R> *
 // PL describes the M = N/2 point complex core, exactly as in k_r2c.
 // ----------------------------------------------------------------------------------------
 struct StftParams {
-    const float *samples;      // [num_samples]
+    const float *samples;      // [batch][num_samples]
     const float *window;       // [wsize] window function values (f32), host-built
-    void *out;                 // MODE_DB: float [frames][M+1];  MODE_COMPLEX: float2 [frames][M+1]
+    void *out;                 // MODE_DB: float [batch][frames][M+1];  MODE_COMPLEX: float2 [batch][frames][M+1]
     const void *tw, *rtw;      // stage tables / W_N^k of the r2c core
-    long frames;
+    long frames;               // per signal: no frame reads samples of another signal
+    long batch, num_samples;   // signals, and the sample stride between them
+    long tiles;                // persistent kernels: tiles of X frames in all, tps per signal: tile t = (t / tps, t % tps)
+    unsigned tps, tps_magic;   // t / tps = (umulhi(t, tps_magic) + t) >> tps_shift for t < 2^31 (stft_tile_signal)
+    int tps_shift;
     int hop, wsize, mode;
     float db_floor;            // gain - range
     float inv_range;           // 1 / range
     float inv_half_n;          // 1 / (N/2)
     unsigned long long *ctr;   // pipelined kernel: zeroed tile counter of this launch
     float lg_a, lg_b;          // fast dB path: value = lg_a * log2(|2 X|^2) + lg_b (host-folded constants)
-    int aligned8;              // `samples` is 8-byte aligned: even hops may use 64-bit loads
+    int aligned8;              // every signal's `samples` row is 8-byte aligned: even hops may use 64-bit loads
     int span_bytes;            // span kernel: shared-memory bytes of one span stage (multiple of 128)
 };
 enum { STFT_MODE_DB = 0, STFT_MODE_COMPLEX = 1 };
+// tile -> (signal, tile within the signal) without a division.  Tiles stay below 2^31: each writes at least one row of
+// N/2 + 1 >= 33 floats, and 2^31 such rows are more than device memory holds.
+inline void stft_tile_magic(StftParams &sp) {
+    int l = 0;
+    while ((1ull << l) < sp.tps) l++;
+    sp.tps_magic = (unsigned)((((1ull << l) - sp.tps) << 32) / sp.tps + 1);      // round-up reciprocal (Granlund-Montgomery)
+    sp.tps_shift = l;
+}
+__device__ __forceinline__ unsigned stft_tile_signal(long tile, const StftParams &sp) {
+    const unsigned t = (unsigned)tile;
+    return (__umulhi(t, sp.tps_magic) + t) >> sp.tps_shift;
+}
 // kernel flavours (template parameter KM): the dB output has a fast path that needs no square root and folds every
 // constant of computeMagnitude / magnitudeToDb / the gain-range normalisation into one FFMA after the MUFU.LG2:
 //   20 log10(|X| c + 1e-10) = 10 log10(|X|^2 c^2) to 1e-6 dB wherever the result is above -150 dB, and everything below
@@ -2283,15 +2299,16 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft(const __grid_constant__
     constexpr int M = PL::N;
     constexpr int LAST = PL::npass() - 1;
     const int xi = threadIdx.x / PL::T, tid = threadIdx.x % PL::T;
-    const long frame = (long)blockIdx.x * X + xi;
-    const bool active = frame < sp.frames;
+    const long frame = (long)blockIdx.x * X + xi;                       // output row: frame f of signal sig
+    const bool active = frame < sp.frames * sp.batch;
+    const long sig = frame / sp.frames, f = frame - sig * sp.frames;
     cx<R> *sm = reinterpret_cast<cx<R> *>(smem_raw) + (size_t)xi * padded_size<PADQ>(M);
     const float2 *tw = reinterpret_cast<const float2 *>(sp.tw);
     const float2 *rtw = reinterpret_cast<const float2 *>(sp.rtw);
     cx<R> x[PL::E];
 
     {   // gather + window + zero-pad: z[p] = (s[off+2p] w[2p], s[off+2p+1] w[2p+1])
-        const float *s = sp.samples + (active ? frame * (long)sp.hop : 0);
+        const float *s = sp.samples + (active ? sig * sp.num_samples + f * (long)sp.hop : 0);
         const bool vec = sp.aligned8 && ((sp.hop | sp.wsize) & 1) == 0;    // aligned base, even hop: frame starts are 8-byte aligned
         static_for<PL::E>([&](auto E_) {
             CIDX(e, E_);
@@ -2337,7 +2354,7 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_pipe(const __grid_const
     const int xi = threadIdx.x / PL::T, tid = threadIdx.x % PL::T;
     const float2 *tw = reinterpret_cast<const float2 *>(sp.tw);
     const float2 *rtw = reinterpret_cast<const float2 *>(sp.rtw);
-    const long tiles = (sp.frames + X - 1) / X;
+    const long tiles = sp.tiles;
 
     if (threadIdx.x == 0) {
         mbar_init(mbar + 0, 1);
@@ -2348,13 +2365,15 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_pipe(const __grid_const
 
     auto issue = [&](long tile, int st) {
         if (threadIdx.x < 32) {
-            const long f0 = tile * X;
+            const unsigned sig = stft_tile_signal(tile, sp);
+            const long f0 = (long)((unsigned)tile - sig * sp.tps) * X;
             const int rows = (sp.frames - f0 < X) ? (int)(sp.frames - f0) : X;
             const uint32_t rowb = (uint32_t)(sp.wsize * sizeof(float));
+            const float *s = sp.samples + (long)sig * sp.num_samples;
             if (threadIdx.x == 0) mbar_expect_tx(mbar + st, rows * rowb);
             __syncwarp();
             for (int r = threadIdx.x; r < rows; r += 32)
-                tma_load_1d(smem_raw + st * BUF + (size_t)r * RSTR * sizeof(float2), sp.samples + (f0 + r) * (long)sp.hop, rowb, mbar + st);
+                tma_load_1d(smem_raw + st * BUF + (size_t)r * RSTR * sizeof(float2), s + (f0 + r) * (long)sp.hop, rowb, mbar + st);
         }
     };
 
@@ -2372,8 +2391,10 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_pipe(const __grid_const
         claim_and_issue<false>(sp.ctr, pending, tiles, slot, st ^ 1, issue);
         mbar_wait(mbar + st, (it >> 1) & 1);
         unsigned char *buf = smem_raw + st * BUF;
-        const long frame = tile * X + xi;
-        const bool active = frame < sp.frames;
+        const unsigned sig = stft_tile_signal(tile, sp);
+        const long f = (long)((unsigned)tile - sig * sp.tps) * X + xi;
+        const bool active = f < sp.frames;
+        const long frame = (long)sig * sp.frames + f;                   // output row
         cx<R> *scratch = reinterpret_cast<cx<R> *>(buf) + (size_t)xi * padded_size<PADQ>(M);
         const float2 *raw = reinterpret_cast<const float2 *>(buf) + (size_t)xi * RSTR;
 
@@ -2475,7 +2496,7 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_span(const __grid_const
     const int xi = threadIdx.x / T, tid = threadIdx.x % T;
     const float2 *tw = reinterpret_cast<const float2 *>(sp.tw);
     const float2 *rtw = reinterpret_cast<const float2 *>(sp.rtw);
-    const long tiles = (sp.frames + X - 1) / X;
+    const long tiles = sp.tiles;
     constexpr int VW = (int)(sizeof(V) / sizeof(float));                 // floats per output bin
     float *gout = reinterpret_cast<float *>(sp.out);
 
@@ -2494,22 +2515,29 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_span(const __grid_const
     }
     __syncthreads();
 
-    auto tile_rows = [&](long tile) { const long f0 = tile * X; return (sp.frames - f0 < X) ? (int)(sp.frames - f0) : X; };
+    // a tile's place, worked out once by the issuing thread and kept per stage in shared memory (not in registers, which
+    // the 32-value plans have none to spare for): {first output row, first frame within its signal}
+    long *geom = slot + 2;
+    auto tile_rows = [&](long f0) { return (sp.frames - f0 < X) ? (int)(sp.frames - f0) : X; };
     // ONE span buffer: a tile's samples are consumed (into registers) at the very start of its iteration, so the next
-    // tile's span is fetched into the same bytes while this tile is computed
-    auto issue = [&](long tile, int) {
+    // tile's span is fetched into the same bytes while this tile is computed.  A span ends at its signal's last frame.
+    auto issue = [&](long tile, int st) {
         if (threadIdx.x == 0) {
-            const uint32_t bytes = (uint32_t)(((long)(tile_rows(tile) - 1) * sp.hop + sp.wsize) * sizeof(float));
+            const unsigned sig = stft_tile_signal(tile, sp);
+            const unsigned f0 = ((unsigned)tile - sig * sp.tps) * X;     // (frames of one signal are far below 2^31)
+            geom[2 * st] = (long)sig * sp.frames + f0;
+            geom[2 * st + 1] = f0;
+            const uint32_t bytes = (uint32_t)((tile_rows(f0) - 1) * sp.hop + sp.wsize) * sizeof(float);
             mbar_expect_tx(mbar, bytes);
-            tma_load_1d(span, sp.samples + tile * X * (long)sp.hop, bytes, mbar);
+            tma_load_1d(span, sp.samples + (long)sig * sp.num_samples + (long)f0 * sp.hop, bytes, mbar);
         }
     };
-    // the result tile of `tile` sits in `work` at the 16-byte phase of its destination
-    auto out_phase = [&](long tile) { return (int)((tile * X * (long)(M + 1) * VW) & 3); };      // in floats
-    auto store_tile = [&](long tile) {
+    // the result tile of stage `st` sits in `work` at the 16-byte phase of its destination
+    auto out_phase = [&](int st) { return (int)((geom[2 * st] * (long)(M + 1) * VW) & 3); };      // in floats
+    auto store_tile = [&](int st) {
         if (threadIdx.x >= 32) return;
-        const long o0 = tile * X * (long)(M + 1) * VW;                   // first float of the tile in the output
-        const int total = tile_rows(tile) * (M + 1) * VW, ph = out_phase(tile);
+        const long o0 = geom[2 * st] * (long)(M + 1) * VW;               // first float of the tile in the output
+        const int total = tile_rows(geom[2 * st + 1]) * (M + 1) * VW, ph = out_phase(st);
         const int head = (4 - ph) & 3;                                   // floats up to the next 16-byte boundary
         const int interior = (total - head) & ~3;
         const float *src = reinterpret_cast<const float *>(work) + ph;
@@ -2526,17 +2554,15 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_span(const __grid_const
     claim_and_issue<false>(sp.ctr, pending, tiles, slot, 0, issue);
     cx<R> x[E];
     unsigned phasebits = 0;
-    long prev_tile = -1;
     for (int it = 0;; it++) {
         const int st = it & 1;
         fence_proxy_async();       // the result tile written below (generic proxy) precedes its bulk store
         __syncthreads();           // slot[st] is published; the result tile of the last iteration is complete
-        if (prev_tile >= 0) store_tile(prev_tile);
+        if (it > 0) store_tile(st ^ 1);                                  // (before the next claim rewrites its geometry)
         const long tile = slot[st];
         if (tile >= tiles) break;
         mbar_wait(mbar, phasebits);
         phasebits ^= 1u;
-        const long frame = tile * X + xi;
         // hop is a multiple of 4 samples: every frame starts on a 16-byte boundary of the span
         const float2 *raw = reinterpret_cast<const float2 *>(span) + (size_t)xi * (sp.hop >> 1);
         static_for<E>([&](auto E_) {
@@ -2559,8 +2585,8 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_span(const __grid_const
         V vk[PER], vm[PER], vh = V();
         stft_values<PL, LAST, KM, V>(x, scratch, rtw, tid, sp, vk, vm, vh);
         __syncthreads();                                                 // every group has read its parked half: `work` becomes the result tile
-        if (frame < sp.frames) {
-            V *orow = reinterpret_cast<V *>(reinterpret_cast<float *>(work) + out_phase(tile)) + (size_t)xi * (M + 1);
+        if (geom[2 * st + 1] + xi < sp.frames) {                         // (frames of the tile's signal)
+            V *orow = reinterpret_cast<V *>(reinterpret_cast<float *>(work) + out_phase(st)) + (size_t)xi * (M + 1);
             static_for<PER>([&](auto I_) {
                 CIDX(i, I_);
                 const int k = tid + i * T;
@@ -2569,7 +2595,6 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_span(const __grid_const
                 if (i == 0 && k == 0) orow[HALF] = vh;
             });
         }
-        prev_tile = tile;
     }
     if (threadIdx.x == 0) bulk_wait_read_all();                         // shared memory must outlive the store that reads it
     claim_epilogue(sp.ctr);
@@ -2590,12 +2615,13 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_span(const __grid_const
 // Shared memory: [X scratch rows, reused as the windowed frames][2 carry buffers of N floats][window, M float2].
 // ----------------------------------------------------------------------------------------
 struct IstftParams {
-    const float2 *spectra;     // [frames][M+1] complex bins
-    float *out;                // [num_samples]
+    const float2 *spectra;     // [batch][frames][M+1] complex bins
+    float *out;                // [batch][num_samples]
     const float *window;       // [wsize] window function values (f32), host-built
     const void *tw, *rtw;      // inverse stage tables / W_N^k of the c2r core
-    long frames, num_samples;
+    long frames, num_samples;  // per signal
     long tile_frames;          // hops of output one CTA owns
+    long tiles;                // CTAs per signal: block b owns tile b % tiles of signal b / tiles
     int hop, wsize, halo;      // halo = ceil(wsize / hop) - 1
     float inv_hop;             // 1 / hop (for small quotients, corrected exactly)
 };
@@ -2624,7 +2650,10 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_istft(const __grid_constant_
         const float2 *w2 = reinterpret_cast<const float2 *>(ip.window);
         for (int p = threadIdx.x; p < M; p += NT) winsm[p] = 2 * p < W ? __ldg(w2 + p) : make_float2(0.0f, 0.0f);
     }
-    const long k0 = (long)blockIdx.x * ip.tile_frames;                   // first frame this CTA owns
+    const long sig = blockIdx.x / ip.tiles;
+    const long k0 = (blockIdx.x - sig * ip.tiles) * ip.tile_frames;      // first frame this CTA owns
+    const float2 *spectra = ip.spectra + sig * ip.frames * (M + 1);
+    float *out = ip.out + sig * ip.num_samples;
     const long a = k0 * H, b = min(a + ip.tile_frames * H, ip.num_samples);
     // sample offset u (from the round's first frame start) = q*H + r, stepped by NT without dividing
     const int tq = threadIdx.x / H, tr = threadIdx.x % H, sq = NT / H, sr = NT % H;
@@ -2638,7 +2667,7 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_istft(const __grid_constant_
             cx<R> *sm = reinterpret_cast<cx<R> *>(work + (size_t)xi * SROW);
             if (f < ip.frames && f * H < b) {
                 // Hermitian pre-process of k_c2r (scale 0.5/M folded in, real parts only at DC and Nyquist)
-                const float2 *in = ip.spectra + f * (M + 1);
+                const float2 *in = spectra + f * (M + 1);
                 static_for<PER>([&](auto I_) {
                     CIDX(i, I_);
                     const int k = tid + i * T;
@@ -2697,7 +2726,7 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_istft(const __grid_constant_
                 float den = 0.0f;
                 const int dlo = (int)min(max(0L, fg - (ip.frames - 1)), (long)dmax + 1);
                 for (int d = (int)min((long)dmax, fg); d >= dlo; d--) { const float w = winf[d * H + r]; den = fmaf(w, w, den); }
-                st_stream(ip.out + gH + u, den >= 1e-11f ? num / den : 0.0f);
+                st_stream(out + gH + u, den >= 1e-11f ? num / den : 0.0f);
             } else {
                 cout[u - (long)X * H] = num;
             }

@@ -222,12 +222,16 @@ template <class PL, int X, int MINB, int PQ = PADQ> struct StftLaunchers {
             case STFT_K_EXACT: k = (const void *)k_stft<PL, X, PQ, MINB, STFT_K_EXACT, true>; break;
             default: k = (const void *)k_stft<PL, X, PQ, MINB, STFT_K_COMPLEX, true>; break;
         }
-        return launch_grid_raw(k, smem, PL::T * X, (sp.frames + X - 1) / X, (void *)&sp, s);
+        return launch_grid_raw(k, smem, PL::T * X, (sp.frames * sp.batch + X - 1) / X, (void *)&sp, s);
     }
     // pipelined variant: XP frames per CTA (>= one warp of threads)
     static constexpr int XP = (PL::T * X >= 128) ? X : 128 / PL::T;
     static constexpr size_t smem_pipe = 2 * real_pipe_buf_bytes<float, PL, PQ, XP, false>() + 64;
-    static cudaError_t launch_pipe(const StftParams &sp, cudaStream_t s) {
+    static cudaError_t launch_pipe(const StftParams &sp0, cudaStream_t s) {
+        StftParams sp = sp0;
+        sp.tps = (unsigned)((sp.frames + XP - 1) / XP);
+        sp.tiles = (long)sp.tps * sp.batch;
+        stft_tile_magic(sp);
         const bool pad = sp.wsize < 2 * PL::N;
         const void *k;
         switch (flavour(sp)) {
@@ -235,7 +239,7 @@ template <class PL, int X, int MINB, int PQ = PADQ> struct StftLaunchers {
             case STFT_K_EXACT: k = (const void *)k_stft_pipe<PL, XP, PQ, MINB, STFT_K_EXACT, true>; break;
             default: k = (const void *)k_stft_pipe<PL, XP, PQ, MINB, STFT_K_COMPLEX, true>; break;
         }
-        return launch_persistent_raw(k, smem_pipe, PL::T * XP, (sp.frames + XP - 1) / XP, (void *)&sp, s);
+        return launch_persistent_raw(k, smem_pipe, PL::T * XP, sp.tiles, (void *)&sp, s);
     }
     static StftVariant make(const char *name) { return StftVariant{name, PL::N, plan_radices<PL>(), &launch, &launch_pipe, nullptr, {}}; }
 };
@@ -250,6 +254,9 @@ template <class PL, int X, int MINB, class SPL, int XS, int SMINB, int SPQ, bool
         const size_t smem = stft_work_bytes<SPL, SPQ, XS>() + span + 128 + sizeof(float2) * SPL::N;      // + mbarriers/slots + window
         if (smem > 200u * 1024u) return cudaErrorInvalidConfiguration;
         sp.span_bytes = (int)span;
+        sp.tps = (unsigned)((sp.frames + XS - 1) / XS);
+        sp.tiles = (long)sp.tps * sp.batch;
+        stft_tile_magic(sp);
         const bool pad = sp.wsize < 2 * SPL::N;
         const void *k;
         switch (StftLaunchers<PL, X, MINB>::flavour(sp)) {
@@ -257,7 +264,7 @@ template <class PL, int X, int MINB, class SPL, int XS, int SMINB, int SPQ, bool
             case STFT_K_EXACT: k = (const void *)k_stft_span<SPL, XS, SPQ, SMINB, STFT_K_EXACT, true>; break;
             default: k = (const void *)k_stft_span<SPL, XS, SPQ, SMINB, STFT_K_COMPLEX, true>; break;
         }
-        return launch_persistent_dyn(k, smem, SPL::T * XS, (sp.frames + XS - 1) / XS, sp, s);
+        return launch_persistent_dyn(k, smem, SPL::T * XS, sp.tiles, sp, s);
     }
     static StftVariant make(const char *name) {
         static_assert(SPL::N == PL::N, "same core size");
