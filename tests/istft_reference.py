@@ -47,12 +47,3 @@ def frames_c2r(spectra, fft_size, irfft=None):
     z[:, -1] = z[:, -1].real
     return np.fft.irfft(z, fft_size, axis=1)
 
-
-def stft_f64(x, fft_size, hop, window_type="hann", zero_padding=1):
-    """Complex STFT in f64 in the library's layout [frames][fft_size/2+1][2] (the f32 window values)."""
-    wsize = fft_size // zero_padding
-    w = window_function(window_type, wsize).astype(np.float32).astype(np.float64)
-    frames = (len(x) - wsize) // hop + 1
-    seg = np.stack([np.asarray(x[f * hop: f * hop + wsize], np.float64) * w for f in range(frames)])
-    z = np.fft.rfft(seg, fft_size, axis=1)
-    return np.stack([z.real, z.imag], axis=-1)

@@ -10,7 +10,8 @@ import pytest
 
 import oracle as om
 from conftest import f32_bound
-from istft_reference import frames_c2r, istft_reference, stft_f64
+from istft_reference import frames_c2r, istft_reference
+from stft_reference import stft_f64
 
 WINDOWS = ("hann", "hamming", "blackman", "blackmanHarris", "rectangular")
 

@@ -9,6 +9,7 @@ import pytest
 
 import oracle as om
 from conftest import f32_bound
+from stft_reference import check
 
 
 def _signal(n, rate=16000.0, seed=0):
@@ -76,8 +77,9 @@ def test_gpu_spectrogram_matches_reference_loop(wf, oracle, n_fft, hop, window, 
 @pytest.mark.gpu
 @pytest.mark.parametrize("n_fft,hop,zp", [(256, 64, 1), (1024, 256, 2)])
 def test_gpu_spectrogram_deep_floor_uses_exact_db(wf, oracle, n_fft, hop, zp):
-    """A floor below -150 dB sees the reference's +1e-10 epsilon (spectrogram.js:60-62): the kernel switches from the
-    fast 10*log10(|X|^2) form to the exact 20*log10(|X|/(N/2) + 1e-10) one.  A signal with exact zeros exercises it."""
+    """A deep floor sees the reference's +1e-10 epsilon (spectrogram.js:60-62): where dropping it would move the output
+    at the floor by more than 1e-6 (floors below about -99 dB at range 80), the kernel switches from the fast
+    10*log10(|X|^2) form to the exact 20*log10(|X|/(N/2) + 1e-10) one.  A signal with exact zeros exercises it."""
     x = _signal(6 * n_fft, seed=7)
     x[: 2 * n_fft] = 0.0                                   # silent frames: magnitude 0 -> -200 dB
     ref = om.spectrogram_reference(x, n_fft, hop, "hann", zp, gain=0.0, range_db=220.0, rfft=oracle.rfft_split_f32)
@@ -112,10 +114,10 @@ def test_gpu_spectrogram_errors_and_long_signal(wf, oracle):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("n_fft,zp", [(256, 1), (256, 2), (512, 1), (512, 2), (1024, 1), (1024, 2), (2048, 1), (4096, 1), (4096, 4), (8192, 1)])
-def test_span_kernel_many_tiles(wf, oracle, monkeypatch, n_fft, zp):
+def test_span_kernel_many_tiles(wf, monkeypatch, n_fft, zp):
     """The span-staged persistent kernel with enough frames that every CTA loops over several tiles and the last tile is
-    ragged: sampled frames against the reference loop, the whole picture against the direct kernel (different core plan,
-    same contract), and bitwise repeatability of the persistent schedule."""
+    ragged: every frame against the f64 STFT, the whole picture against the direct kernel (different core plan, same
+    contract), and bitwise repeatability of the persistent schedule."""
     hop = n_fft // zp // 4
     frames_wanted = 9001 if n_fft <= 1024 else 3001
     ns = (frames_wanted - 1) * hop + n_fft // zp + 3
@@ -130,11 +132,7 @@ def test_span_kernel_many_tiles(wf, oracle, monkeypatch, n_fft, zp):
     g, d = got["data"].reshape(f, b), direct["data"].reshape(f, b)
     assert np.array_equal(g, again["data"].reshape(f, b))
     assert np.max(np.abs(g - d)) < 2e-4
-    w = n_fft // zp
-    for fr in (0, 1, 7, 8, f // 2, f - 9, f - 2, f - 1):
-        ref = om.spectrogram_reference(x[fr * hop: fr * hop + w], n_fft, hop, "hann", zp, gain=-3.0, range_db=75.0,
-                                       rfft=oracle.rfft_split_f32)
-        assert np.max(np.abs(g[fr] - ref[0])) < 2e-4, fr
+    check(g, x, n_fft, hop, "hann", zp, "db", gain=-3.0, range_db=75.0)
 
 
 @pytest.mark.gpu

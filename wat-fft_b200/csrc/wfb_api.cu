@@ -1215,7 +1215,8 @@ int wfb_stft_exec_device(wfb_stft *st, const float *d_samples, void *d_out, void
     sp.lg_a = 3.0102999566398120f * st->inv_range;
     sp.lg_b = sp.lg_a * (2.0f * log2f(sp.inv_half_n) - 2.0f) - st->db_floor * st->inv_range;
     // frames are TMA-copyable when their starts are 16-byte aligned (hop % 4 == 0, aligned base)
-    static const int pipe_min = [] { const char *e = getenv("WFB_STFT_PIPE_MIN_N"); return e ? atoi(e) : 8192; }();
+    const char *pipe_env = getenv("WFB_STFT_PIPE_MIN_N");       // (read per call, like WFB_STFT_SPAN below)
+    const int pipe_min = pipe_env ? atoi(pipe_env) : 8192;
     const bool pipe = st->fft_size >= pipe_min && st->hop % 4 == 0 && st->wsize % 4 == 0 && rows16;
     cudaStream_t cs = stream ? (cudaStream_t)stream : st->stream;
     // span kernel: whole tiles of overlapping frames as one bulk copy (16-byte aligned frame starts and sizes)

@@ -2228,8 +2228,10 @@ __device__ __forceinline__ unsigned stft_tile_signal(long tile, const StftParams
 }
 // kernel flavours (template parameter KM): the dB output has a fast path that needs no square root and folds every
 // constant of computeMagnitude / magnitudeToDb / the gain-range normalisation into one FFMA after the MUFU.LG2:
-//   20 log10(|X| c + 1e-10) = 10 log10(|X|^2 c^2) to 1e-6 dB wherever the result is above -150 dB, and everything below
-//   the floor (gain - range) clamps to 0 either way; a floor deeper than -150 dB selects the exact form.
+//   10 log10(|X|^2 c^2) = 20 log10(|X| c + 1e-10) - 20 log10(1 + 1e-10 / (|X| c)): below by 1e-6 dB at -61 dB, 8.7e-5 dB
+//   at -100 dB and ten times more per 20 dB deeper.  Everything below the floor (gain - range) clamps to 0 either way, so the error
+//   that counts is the one at the floor; StftLaunchers::flavour takes the fast form only where it is at most 1e-6 of the
+//   normalised output there, and the exact form below that.
 enum { STFT_K_FAST = 0, STFT_K_EXACT = 1, STFT_K_COMPLEX = 2 };
 
 __device__ __forceinline__ float stft_db(float re, float im, const StftParams &sp) {

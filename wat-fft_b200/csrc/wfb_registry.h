@@ -208,11 +208,14 @@ cudaError_t launch_grid_raw(const void *kernel, size_t smem, int threads, long c
 const std::vector<StftVariant> &variants_stft();
 template <class PL, int X, int MINB, int PQ = PADQ> struct StftLaunchers {
     static constexpr size_t smem = sizeof(cx<float>) * (size_t)padded_size<PQ>(PL::N) * X;
-    // kernel flavour: fast dB (floor above -150 dB) / exact dB / complex output; the unpadded fast-dB case (window =
-    // FFT size, the spectrogram default) gets its own instantiation without the per-element bound check
+    // kernel flavour: fast dB / exact dB / complex output; the unpadded fast-dB case (window = FFT size, the spectrogram
+    // default) gets its own instantiation without the per-element bound check.  The fast form drops the +1e-10 of
+    // magnitudeToDb, which lowers a value by 20 log10(1 + 1e-10 / (|X| c)) dB, the most at the floor (gain - range): it
+    // runs only where that is at most 1e-6 of the [0, 1] output there (floors down to about -99 dB at range 80)
     static int flavour(const StftParams &sp) {
         if (sp.mode == STFT_MODE_COMPLEX) return STFT_K_COMPLEX;
-        return sp.db_floor >= -150.0f ? STFT_K_FAST : STFT_K_EXACT;
+        const double worst = 20.0 * log10(1.0 + 1e-10 * pow(10.0, -(double)sp.db_floor / 20.0)) * (double)sp.inv_range;
+        return worst > 1e-6 ? STFT_K_EXACT : STFT_K_FAST;
     }
     static cudaError_t launch(const StftParams &sp, cudaStream_t s) {
         const bool pad = sp.wsize < 2 * PL::N;
