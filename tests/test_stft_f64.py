@@ -52,7 +52,7 @@ def _record(kernel, flavour, ratio):
 
 
 def _exact_db(gain, range_db):
-    """Whether the library takes the exact dB form (StftLaunchers::flavour): where the fast form's dropped +1e-10 would
+    """Whether the library takes the exact dB form (stft_flavour): where the fast form's dropped +1e-10 would
     lower the output at the floor by more than 1e-6."""
     floor = np.float32(gain) - np.float32(range_db)
     inv_range = float(np.float32(1.0) / np.float32(range_db))

@@ -40,57 +40,11 @@ static int cuda_fail(cudaError_t e, const char *what) {
 // kernel launch helpers (one launch counter and one attribute cache for the whole library)
 // ----------------------------------------------------------------------------------------
 static std::mutex g_mu;
-static std::map<std::pair<int, const void *>, int> g_resident;   // (device, kernel) -> resident CTAs
-
-static cudaError_t configure(const void *kernel, size_t smem, int threads, int *resident) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    std::lock_guard<std::mutex> lock(g_mu);
-    auto key = std::make_pair(dev, kernel);
-    auto it = g_resident.find(key);
-    if (it == g_resident.end()) {
-        // the dynamic-smem attribute is per (device, function); set it once for each pair
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        // NOTE: forcing cudaSharedmemCarveoutMaxShared was measured (gpurun sweep9) to LOSE 5-15 %: it shrinks
-        // L1, which the twiddle tables and the direct-load kernels live in.  The driver's default split stays.
-        int per_sm = 0, sms = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem);
-        if (e != cudaSuccess) return e;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if (per_sm < 1) per_sm = 1;
-        it = g_resident.emplace(key, per_sm * sms).first;
-    }
-    *resident = it->second;
-    return cudaSuccess;
-}
-
-cudaError_t launch_grid(const void *kernel, size_t smem, int threads, long ctas, const KParams &p, cudaStream_t s) {
-    if (!kernel) return cudaErrorInvalidDeviceFunction;
-    int resident;
-    cudaError_t e = configure(kernel, smem, threads, &resident);
-    if (e != cudaSuccess) return e;
-    void *args[] = {(void *)&p};
-    e = cudaLaunchKernel(kernel, dim3((unsigned)ctas), dim3(threads), args, smem, s);
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return e != cudaSuccess ? e : cudaGetLastError();
-}
-
-cudaError_t launch_grid_raw(const void *kernel, size_t smem, int threads, long ctas, void *params, cudaStream_t s) {
-    if (!kernel) return cudaErrorInvalidDeviceFunction;
-    int resident;
-    cudaError_t e = configure(kernel, smem, threads, &resident);
-    if (e != cudaSuccess) return e;
-    void *args[] = {params};
-    e = cudaLaunchKernel(kernel, dim3((unsigned)ctas), dim3(threads), args, smem, s);
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return e != cudaSuccess ? e : cudaGetLastError();
-}
 
 // Per-launch tile counters of the persistent kernels: a ring of {claims, departures} pairs per device, zeroed once
 // when the ring is created.  Every kernel leaves its pair at zero again (claim_epilogue), so nothing has to be cleared
 // between launches; a pair would only be reused while still live if 4096 persistent launches were outstanding at once.
-static cudaError_t next_counter(cudaStream_t, unsigned long long **out) {
+static cudaError_t next_counter(unsigned long long **out) {
     enum { RING = 4096 };
     static std::map<int, unsigned long long *> rings;
     static std::map<int, unsigned> heads;
@@ -118,69 +72,43 @@ static cudaError_t next_counter(cudaStream_t, unsigned long long **out) {
     return cudaSuccess;
 }
 
-cudaError_t launch_persistent_raw(const void *kernel, size_t smem, int threads, long work_items, void *params, cudaStream_t s) {
+cudaError_t launch(const void *kernel, size_t smem, size_t smem_attr, int threads, long work_items, void *params,
+                   unsigned long long **ctr, cudaStream_t s) {
     if (!kernel) return cudaErrorInvalidDeviceFunction;
-    int resident;
-    cudaError_t e = configure(kernel, smem, threads, &resident);
-    if (e != cudaSuccess) return e;
-    StftParams sp = *static_cast<const StftParams *>(params);      // the only raw-parameter persistent kernel
-    if ((e = next_counter(s, &sp.ctr)) != cudaSuccess) return e;
-    long grid = work_items < resident ? work_items : resident;
-    void *args[] = {&sp};
-    e = cudaLaunchKernel(kernel, dim3((unsigned)grid), dim3(threads), args, smem, s);
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return e != cudaSuccess ? e : cudaGetLastError();
-}
-
-// persistent launch with per-call dynamic shared memory (k_stft_span): the opt-in limit is raised once per kernel, the
-// resident-CTA count is cached per (device, kernel, bytes)
-cudaError_t launch_persistent_dyn(const void *kernel, size_t smem, int threads, long work_items, const StftParams &sp0, cudaStream_t s) {
-    if (!kernel) return cudaErrorInvalidDeviceFunction;
-    static std::map<std::pair<std::pair<int, const void *>, size_t>, int> cache;
-    static std::set<std::pair<int, const void *>> raised;
-    int dev = 0, resident = 0;
+    static std::set<std::pair<int, const void *>> configured;
+    static std::map<std::pair<std::pair<int, const void *>, size_t>, int> resident;    // (device, kernel, smem) -> CTAs on the GPU
+    int dev = 0, ctas = 0;
     cudaGetDevice(&dev);
     {
         std::lock_guard<std::mutex> lock(g_mu);
         const auto fk = std::make_pair(dev, kernel);
-        if (!raised.count(fk)) {
-            cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        if (!configured.count(fk)) {
+            // the dynamic-smem attribute is per (device, function); set it once for each pair
+            cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_attr);
             if (e != cudaSuccess) return e;
-            raised.insert(fk);
+            // NOTE: forcing cudaSharedmemCarveoutMaxShared was measured (gpurun sweep9) to LOSE 5-15 %: it shrinks
+            // L1, which the twiddle tables and the direct-load kernels live in.  The driver's default split stays.
+            configured.insert(fk);
         }
-        const auto key = std::make_pair(fk, smem);
-        auto it = cache.find(key);
-        if (it == cache.end()) {
+        auto it = resident.find(std::make_pair(fk, smem));
+        if (it == resident.end()) {
             int per_sm = 0, sms = 0;
             cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem);
             if (e != cudaSuccess) return e;
+            if (per_sm < 1) return cudaErrorInvalidConfiguration;      // not even one CTA fits an SM
             cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-            if (per_sm < 1) return cudaErrorInvalidConfiguration;
-            it = cache.emplace(key, per_sm * sms).first;
+            it = resident.emplace(std::make_pair(fk, smem), per_sm * sms).first;
         }
-        resident = it->second;
+        ctas = it->second;
     }
-    StftParams sp = sp0;
-    cudaError_t e = next_counter(s, &sp.ctr);
-    if (e != cudaSuccess) return e;
-    long grid = work_items < resident ? work_items : resident;
-    void *args[] = {&sp};
-    e = cudaLaunchKernel(kernel, dim3((unsigned)grid), dim3(threads), args, smem, s);
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return e != cudaSuccess ? e : cudaGetLastError();
-}
-
-// persistent kernels: grid = min(work items, CTAs resident on the whole GPU)
-cudaError_t launch_persistent(const void *kernel, size_t smem, int threads, long work_items, const KParams &p, cudaStream_t s) {
-    if (!kernel) return cudaErrorInvalidDeviceFunction;
-    int resident;
-    cudaError_t e = configure(kernel, smem, threads, &resident);
-    if (e != cudaSuccess) return e;
-    KParams q = p;
-    if ((e = next_counter(s, &q.ctr)) != cudaSuccess) return e;
-    long grid = work_items < resident ? work_items : resident;
-    void *args[] = {&q};
-    e = cudaLaunchKernel(kernel, dim3((unsigned)grid), dim3(threads), args, smem, s);
+    long grid = work_items;
+    if (ctr) {
+        cudaError_t e = next_counter(ctr);
+        if (e != cudaSuccess) return e;
+        grid = std::min<long>(work_items, ctas);
+    }
+    void *args[] = {params};
+    cudaError_t e = cudaLaunchKernel(kernel, dim3((unsigned)grid), dim3(threads), args, smem, s);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return e != cudaSuccess ? e : cudaGetLastError();
 }
@@ -382,6 +310,27 @@ int wfb_reference_twiddles(int flavour, int n, int count, void *re, void *im) {
 
 }  // extern "C"
 
+// Base-table flavour of an f32 scalar-lane core whose reference table is `reference`.  Kernels that DERIVE w2 = w1^2,
+// w3 = w1*w2 in registers (f32 scalar lanes, core >= WFB_DERIVE_MIN_N: derive_tw in wfb_kernels.cuh) square and cube
+// whatever error w1 carries.  The reference's f32 table is a 6-term Taylor series good to ~5e-7; derived from it, w3 is off
+// by 1.5e-6 and N = 4096 misses the reference's own absolute threshold (tests/fft_f32_dual.test.js:83-86: 2.6e-4 against
+// 2.0e-4).  So those kernels get CORRECTLY ROUNDED w1 (error 6e-8): the derived factors are then more accurate than the
+// reference's looked-up ones, and the f32 contract is tolerance-based.
+static int scalar_f32_flavour(int m, int reference) { return m >= WFB_DERIVE_MIN_N ? TW_EXACT : reference; }
+
+// rfft_split's fused radix-8 opening uses exact W_8 constants for group 1 of the l = 2 stage
+// (fft_split_native_f32.wat:1199-1371): patched into the forward stage table `fwd` of an f32 r2c core
+static void w8_opening(int m, const std::vector<int> &radices, std::vector<float> &fwd) {
+    if (!((ilog2(m) & 1) && m >= 32 && radices.size() >= 2 && radices[0] == 2 && radices[1] == 4)) return;
+    const float c = float(0.7071067811865476);
+    const size_t off = 2 * 1;               // skip the radix-2 stage's single entry (re,im)
+    const int l = 2;
+    const float w[3][2] = {{c, -c}, {0.0f, -1.0f}, {-c, -c}};
+    for (int mm = 0; mm < 3; mm++) { fwd[off + 2 * (mm * l + 1)] = w[mm][0]; fwd[off + 2 * (mm * l + 1) + 1] = w[mm][1]; }
+}
+
+static size_t up256(size_t b) { return (b + 255) / 256 * 256; }
+
 // builds forward / inverse stage tables for one variant and uploads them
 template <typename R>
 static int upload_tables(wfb_plan *pl, int vi) {
@@ -389,28 +338,15 @@ static int upload_tables(wfb_plan *pl, int vi) {
     const int m = v.core_n;
     int flavour;
     if (sizeof(R) == 8) flavour = (m == 16 || m <= 4) ? TW_EXACT : TW_F64;
-    else if (pl->kind == WFB_C2C && pl->layout == WFB_INTERLEAVED) flavour = (m <= 16) ? TW_EXACT : TW_F32_DUAL;
-    else flavour = TW_F32_SPLIT;
-    // Kernels that DERIVE w2 = w1^2, w3 = w1*w2 in registers (f32 scalar lanes, core >= WFB_DERIVE_MIN_N: derive_tw in
-    // wfb_kernels.cuh) square and cube whatever error w1 carries.  The reference's f32 table is a 6-term Taylor series good to
-    // ~5e-7; derived from it, w3 is off by 1.5e-6 and N = 4096 misses the reference's own absolute threshold
-    // (tests/fft_f32_dual.test.js:83-86: 2.6e-4 against 2.0e-4).  So those kernels get CORRECTLY ROUNDED w1 (error 6e-8): the
-    // derived factors are then more accurate than the reference's looked-up ones, and the f32 contract is tolerance-based.
-    if (sizeof(R) == 4 && v.lanes == 1 && m >= WFB_DERIVE_MIN_N) flavour = TW_EXACT;
+    else {
+        flavour = (pl->kind == WFB_C2C && pl->layout == WFB_INTERLEAVED) ? (m <= 16 ? TW_EXACT : TW_F32_DUAL) : TW_F32_SPLIT;
+        if (v.lanes == 1) flavour = scalar_f32_flavour(m, flavour);
+    }
     std::vector<R> bre, bim, fwd, inv;
     base_twiddles<R>(flavour, m, m, bre, bim);
     stage_tables<R>(v.radices, m, bre, bim, false, fwd);
     stage_tables<R>(v.radices, m, bre, bim, true, inv);
-    if (pl->kind == WFB_R2C && sizeof(R) == 4 && (ilog2(m) & 1) && m >= 32 && v.radices.size() >= 2 &&
-        v.radices[0] == 2 && v.radices[1] == 4) {
-        // rfft_split's fused radix-8 opening uses exact W_8 constants for group 1 of the l = 2 stage
-        // (fft_split_native_f32.wat:1199-1371); forward table only.
-        const R c = R(0.7071067811865476);
-        size_t off = 2 * 1;                 // skip the radix-2 stage's single entry (re,im)
-        const int l = 2;
-        R w[3][2] = {{c, -c}, {R(0), R(-1)}, {-c, -c}};
-        for (int mm = 0; mm < 3; mm++) { fwd[off + 2 * (mm * l + 1)] = w[mm][0]; fwd[off + 2 * (mm * l + 1) + 1] = w[mm][1]; }
-    }
+    if constexpr (sizeof(R) == 4) if (pl->kind == WFB_R2C) w8_opening(m, v.radices, fwd);
     if (fwd.empty()) { fwd.assign(2, R(0)); inv.assign(2, R(0)); }
     // packed-lane kernels read entries as (re, re, im, im)
     auto widen = [&](std::vector<R> &t) {
@@ -438,7 +374,6 @@ static int upload_tables(wfb_plan *pl, int vi) {
         widen(packed);
     }
     // one allocation and one copy per variant: [forward | inverse | W_n^k], each 256-byte aligned
-    auto up256 = [](size_t b) { return (b + 255) / 256 * 256; };
     const size_t bf = up256(fwd.size() * sizeof(R)), bi = up256(inv.size() * sizeof(R)), br = up256(packed.size() * sizeof(R));
     std::vector<unsigned char> blob(bf + bi + br, 0);
     memcpy(blob.data(), fwd.data(), fwd.size() * sizeof(R));
@@ -1064,9 +999,10 @@ int wfb_pcie_probe(int device, size_t bytes, int iters, double gbs[4]) {
 // batched STFT front-end
 // ----------------------------------------------------------------------------------------
 struct wfb_stft {
-    int fft_size, wsize, hop, mode, device, flags;
+    int fft_size, wsize, hop, mode, window, device, flags;
     long num_samples, frames, batch;   // frames per signal; batch signals of num_samples each
     const StftVariant *variant;
+    void *d_tables;                    // the one allocation d_tw / d_tw_span / d_rtw / d_window point into
     void *d_tw, *d_tw_span, *d_rtw, *d_window, *d_samples, *d_out;
     void *h_samples, *h_out;
     size_t in_bytes, out_bytes;        // whole batch
@@ -1096,29 +1032,31 @@ static int stft_init(wfb_stft *st) {
     const int n = st->fft_size, m = n / 2;
     const StftVariant &v = *st->variant;
     std::vector<float> bre, bim, fwd, fwd_span, rre, rim, packed, win(st->wsize);
-    base_twiddles<float>(m >= WFB_DERIVE_MIN_N ? TW_EXACT : TW_F32_SPLIT, m, m, bre, bim);      // (derived w2, w3: see upload_tables)
+    base_twiddles<float>(scalar_f32_flavour(m, TW_F32_SPLIT), m, m, bre, bim);
     auto tables = [&](const std::vector<int> &radices, std::vector<float> &t) {
         stage_tables<float>(radices, m, bre, bim, false, t);
-        if ((ilog2(m) & 1) && m >= 32 && radices.size() >= 2 && radices[0] == 2 && radices[1] == 4) {
-            const float c = 0.7071067811865476f;      // rfft_split's exact W_8 opening (see upload_tables)
-            const float w[3][2] = {{c, -c}, {0.f, -1.f}, {-c, -c}};
-            for (int mm = 0; mm < 3; mm++) { t[2 + 2 * (mm * 2 + 1)] = w[mm][0]; t[2 + 2 * (mm * 2 + 1) + 1] = w[mm][1]; }
-        }
+        w8_opening(m, radices, t);
     };
     tables(v.radices, fwd);
     if (!v.span_radices.empty() && v.span_radices != v.radices) tables(v.span_radices, fwd_span);   // the span kernel's core plan groups the stages differently
     base_twiddles<float>(TW_F32_SPLIT, n, m + 1, rre, rim);
     for (int k = 0; k <= m; k++) { packed.push_back(rre[k]); packed.push_back(rim[k]); }
-    for (int i = 0; i < st->wsize; i++) win[i] = (float)window_value(st->mode >> 8, i, st->wsize);
-    auto up = [&](void **d, const std::vector<float> &h) -> int {
-        CK(cudaMalloc(d, h.size() * sizeof(float)));
-        CK(cudaMemcpy(*d, h.data(), h.size() * sizeof(float), cudaMemcpyHostToDevice));
-        return WFB_OK;
-    };
-    int rc;
-    if ((rc = up(&st->d_tw, fwd)) || (rc = up(&st->d_rtw, packed)) || (rc = up(&st->d_window, win))) return rc;
-    if (!fwd_span.empty() && (rc = up(&st->d_tw_span, fwd_span))) return rc;
-    CK(cudaDeviceSynchronize());      // the uploads above ran on the legacy stream; the plan's stream does not order against it
+    for (int i = 0; i < st->wsize; i++) win[i] = (float)window_value(st->window, i, st->wsize);
+    // one allocation and one copy: [forward | span forward | W_n^k | window], each 256-byte aligned
+    const std::vector<float> *sec[4] = {&fwd, &fwd_span, &packed, &win};
+    size_t off[5] = {0};
+    for (int i = 0; i < 4; i++) off[i + 1] = off[i] + up256(sec[i]->size() * sizeof(float));
+    std::vector<unsigned char> blob(off[4], 0);
+    for (int i = 0; i < 4; i++) if (!sec[i]->empty()) memcpy(blob.data() + off[i], sec[i]->data(), sec[i]->size() * sizeof(float));
+    CK(cudaMalloc(&st->d_tables, blob.size()));
+    // stream-ordered on the handle's stream and completed here: launches on ANY stream may follow
+    CK(cudaMemcpyAsync(st->d_tables, blob.data(), blob.size(), cudaMemcpyHostToDevice, st->stream));
+    CK(cudaStreamSynchronize(st->stream));
+    unsigned char *d = (unsigned char *)st->d_tables;
+    st->d_tw = d;
+    st->d_tw_span = fwd_span.empty() ? nullptr : d + off[1];
+    st->d_rtw = d + off[2];
+    st->d_window = d + off[3];
     if (!(st->flags & WFB_PLAN_NO_DEVICE_BUFFERS)) {
         if (cudaMalloc(&st->d_samples, st->in_bytes) != cudaSuccess) { cudaGetLastError(); return WFB_ERR_ALLOC; }
         if (cudaMalloc(&st->d_out, st->out_bytes) != cudaSuccess) { cudaGetLastError(); return WFB_ERR_ALLOC; }
@@ -1130,6 +1068,24 @@ static int stft_init(wfb_stft *st) {
         memset(st->h_out, 0, st->out_bytes);
     }
     return WFB_OK;
+}
+
+// The STFT kernel for these pointers (STFT_DIRECT, STFT_SPAN or STFT_PIPE).  The bulk-copy kernels (span, pipe) copy
+// frames or tile spans into shared memory, so frame starts and sizes must be 16-byte aligned in every signal.
+static int stft_route(const wfb_stft *st, const float *d_samples, const void *d_out) {
+    const StftVariant &v = *st->variant;
+    const bool rows16 = ((uintptr_t)d_samples % 16) == 0 && (st->batch == 1 || st->num_samples % 4 == 0);
+    const bool bulk = st->hop % 4 == 0 && st->wsize % 4 == 0 && rows16;
+    // span kernel: whole tiles of overlapping frames as one bulk copy in, and one bulk store out; very large hops make
+    // the span too large for shared memory
+    const char *span_env = getenv("WFB_STFT_SPAN");             // (read per call: tests and A/B runs flip it)
+    const bool span_on = span_env ? atoi(span_env) != 0 : v.span_default;      // WFB_STFT_SPAN=1 forces, =0 forbids
+    if (span_on && v.launch[STFT_SPAN] && bulk && ((uintptr_t)d_out % 16) == 0 &&
+        v.span_fixed_bytes + stft_span_bytes(v.span_frames, st->hop, st->wsize) <= STFT_SPAN_SMEM_MAX)
+        return STFT_SPAN;
+    const char *pipe_env = getenv("WFB_STFT_PIPE_MIN_N");       // (read per call, like WFB_STFT_SPAN)
+    const int pipe_min = pipe_env ? atoi(pipe_env) : 8192;
+    return st->fft_size >= pipe_min && bulk ? STFT_PIPE : STFT_DIRECT;
 }
 
 extern "C" {
@@ -1160,7 +1116,8 @@ wfb_stft *wfb_stft_create_ex(int fft_size, int zero_padding, int hop, int window
     if (*err) return nullptr;
     wfb_stft *st = new wfb_stft();
     st->fft_size = fft_size; st->wsize = wsize; st->hop = hop; st->device = device; st->flags = flags;
-    st->mode = mode | (window_type << 8);
+    st->mode = mode;
+    st->window = window_type;
     st->num_samples = num_samples;
     st->frames = (long)frames;
     st->batch = batch;
@@ -1180,7 +1137,7 @@ void wfb_stft_destroy(wfb_stft *st) {
     if (!st) return;
     cudaSetDevice(st->device);
     if (st->stream) { cudaStreamSynchronize(st->stream); cudaStreamDestroy(st->stream); }
-    void *d[] = {st->d_tw, st->d_tw_span, st->d_rtw, st->d_window, st->d_samples, st->d_out, st->d_tw_inv};
+    void *d[] = {st->d_tables, st->d_samples, st->d_out, st->d_tw_inv};
     for (void *p : d) if (p) cudaFree(p);
     if (st->inv_ready) cudaEventDestroy(st->inv_ready);
     if (st->h_samples) cudaFreeHost(st->h_samples);
@@ -1202,33 +1159,20 @@ int wfb_stft_exec_device(wfb_stft *st, const float *d_samples, void *d_out, void
     StftParams sp;
     sp.samples = d_samples; sp.window = (const float *)st->d_window; sp.out = d_out;
     sp.tw = st->d_tw; sp.rtw = st->d_rtw;
-    sp.frames = st->frames; sp.batch = st->batch; sp.num_samples = st->num_samples; sp.hop = st->hop; sp.wsize = st->wsize; sp.mode = st->mode & 0xFF;
+    sp.frames = st->frames; sp.batch = st->batch; sp.num_samples = st->num_samples; sp.hop = st->hop; sp.wsize = st->wsize; sp.mode = st->mode;
     sp.db_floor = st->db_floor; sp.inv_range = st->inv_range; sp.inv_half_n = 2.0f / (float)st->fft_size;
     sp.ctr = nullptr;
     sp.span_bytes = 0;
     sp.tiles = 0; sp.tps = sp.tps_magic = 0; sp.tps_shift = 0;      // (set by the persistent kernels' launchers)
     // a caller's pointer may be any float address (scalar loads then); the rows of a batch keep the base's alignment only
-    // when num_samples is a multiple of 2 (8 bytes) or 4 (16 bytes, the bulk-copy kernels)
+    // when num_samples is a multiple of 2 (8 bytes) or 4 (16 bytes, the bulk-copy kernels: stft_route)
     sp.aligned8 = ((uintptr_t)d_samples % 8) == 0 && (st->batch == 1 || st->num_samples % 2 == 0);
-    const bool rows16 = ((uintptr_t)d_samples % 16) == 0 && (st->batch == 1 || st->num_samples % 4 == 0);
     // fast dB path: v = lg_a * log2(|2 X|^2) + lg_b  ==  (10 log10(|X|^2 c^2) - floor) / range,  c = 2 / fft_size
     sp.lg_a = 3.0102999566398120f * st->inv_range;
     sp.lg_b = sp.lg_a * (2.0f * log2f(sp.inv_half_n) - 2.0f) - st->db_floor * st->inv_range;
-    // frames are TMA-copyable when their starts are 16-byte aligned (hop % 4 == 0, aligned base)
-    const char *pipe_env = getenv("WFB_STFT_PIPE_MIN_N");       // (read per call, like WFB_STFT_SPAN below)
-    const int pipe_min = pipe_env ? atoi(pipe_env) : 8192;
-    const bool pipe = st->fft_size >= pipe_min && st->hop % 4 == 0 && st->wsize % 4 == 0 && rows16;
-    cudaStream_t cs = stream ? (cudaStream_t)stream : st->stream;
-    // span kernel: whole tiles of overlapping frames as one bulk copy (16-byte aligned frame starts and sizes)
-    const char *span_env = getenv("WFB_STFT_SPAN");             // (read per call: tests and A/B runs flip it)
-    const bool span_on = span_env ? atoi(span_env) != 0 : st->variant->span_default;      // WFB_STFT_SPAN=1 forces, =0 forbids
-    cudaError_t e = cudaErrorInvalidConfiguration;
-    if (span_on && st->variant->launch_span && st->hop % 4 == 0 && st->wsize % 4 == 0 && rows16 && ((uintptr_t)d_out % 16) == 0) {
-        StftParams ss = sp;
-        if (st->d_tw_span) ss.tw = st->d_tw_span;
-        e = st->variant->launch_span(ss, cs);
-    }
-    if (e == cudaErrorInvalidConfiguration) { cudaGetLastError(); e = (pipe ? st->variant->launch_pipe : st->variant->launch)(sp, cs); }
+    const int route = stft_route(st, d_samples, d_out);
+    if (route == STFT_SPAN && st->d_tw_span) sp.tw = st->d_tw_span;
+    cudaError_t e = st->variant->launch[route](sp, stream ? (cudaStream_t)stream : st->stream);
     if (e != cudaSuccess) return cuda_fail(e, "stft launch");
     return WFB_OK;
 }
@@ -1254,7 +1198,7 @@ static int stft_inverse_tables(wfb_stft *st, cudaStream_t cs) {
     }
     const int m = st->fft_size / 2;
     std::vector<float> bre, bim, inv;
-    base_twiddles<float>(m >= WFB_DERIVE_MIN_N ? TW_EXACT : TW_F32_SPLIT, m, m, bre, bim);
+    base_twiddles<float>(scalar_f32_flavour(m, TW_F32_SPLIT), m, m, bre, bim);
     stage_tables<float>(st->inv_variant->radices, m, bre, bim, true, inv);
     if (inv.empty()) inv.assign(2, 0.0f);
     void *d = nullptr;
@@ -1269,7 +1213,7 @@ static int stft_inverse_tables(wfb_stft *st, cudaStream_t cs) {
 
 int wfb_stft_exec_inverse_device(wfb_stft *st, const void *d_spectra, float *d_samples, void *stream) {
     if (!st || !d_spectra || !d_samples) return WFB_ERR_BAD_ARG;
-    if ((st->mode & 0xFF) != WFB_STFT_COMPLEX) return WFB_ERR_UNSUPPORTED;      // dB magnitudes have no inverse
+    if (st->mode != WFB_STFT_COMPLEX) return WFB_ERR_UNSUPPORTED;      // dB magnitudes have no inverse
     if (((uintptr_t)d_spectra % 8) != 0) return WFB_ERR_BAD_ARG;
     const uintptr_t s0 = (uintptr_t)d_spectra, s1 = s0 + st->out_bytes;
     const uintptr_t x0 = (uintptr_t)d_samples, x1 = x0 + st->in_bytes;
@@ -1300,7 +1244,7 @@ int wfb_stft_exec_inverse_device(wfb_stft *st, const void *d_spectra, float *d_s
 
 int wfb_stft_exec_inverse(wfb_stft *st, int flags) {
     if (!st || !st->d_samples) return WFB_ERR_BAD_ARG;
-    if ((st->mode & 0xFF) != WFB_STFT_COMPLEX) return WFB_ERR_UNSUPPORTED;
+    if (st->mode != WFB_STFT_COMPLEX) return WFB_ERR_UNSUPPORTED;
     if ((flags & (WFB_STAGE_H2D | WFB_STAGE_D2H)) && !st->h_out) return WFB_ERR_NO_HOST_BUFFERS;
     CK(cudaSetDevice(st->device));
     if (flags & WFB_STAGE_H2D) CK(cudaMemcpyAsync(st->d_out, st->h_out, st->out_bytes, cudaMemcpyHostToDevice, st->stream));

@@ -2230,9 +2230,10 @@ __device__ __forceinline__ unsigned stft_tile_signal(long tile, const StftParams
 // constant of computeMagnitude / magnitudeToDb / the gain-range normalisation into one FFMA after the MUFU.LG2:
 //   10 log10(|X|^2 c^2) = 20 log10(|X| c + 1e-10) - 20 log10(1 + 1e-10 / (|X| c)): below by 1e-6 dB at -61 dB, 8.7e-5 dB
 //   at -100 dB and ten times more per 20 dB deeper.  Everything below the floor (gain - range) clamps to 0 either way, so the error
-//   that counts is the one at the floor; StftLaunchers::flavour takes the fast form only where it is at most 1e-6 of the
+//   that counts is the one at the floor; stft_flavour takes the fast form only where it is at most 1e-6 of the
 //   normalised output there, and the exact form below that.
 enum { STFT_K_FAST = 0, STFT_K_EXACT = 1, STFT_K_COMPLEX = 2 };
+template <int KM> using stft_value_t = typename std::conditional<KM == STFT_K_COMPLEX, float2, float>::type;   // one output bin
 
 __device__ __forceinline__ float stft_db(float re, float im, const StftParams &sp) {
     // computeMagnitude + magnitudeToDb + normalisation (spectrogram.js:78-96, :343-352)
@@ -2248,28 +2249,29 @@ __device__ __forceinline__ float stft_db_fast(cx<float> x2, const StftParams &sp
     return fminf(1.0f, fmaxf(0.0f, v));
 }
 
-// Hermitian post-process + output stage shared by the two STFT kernels.  `park` holds the upper half of the core's
-// outputs (park_upper_half); Z[k] for k < M/2 is the thread's own register value.
-template <class PL, int LAST, int KM>
-__device__ __forceinline__ void stft_post(const cx<float> (&x)[PL::E], const cx<float> *park, const float2 *rtw, int tid,
-                                          long frame, const StftParams &sp) {
+// Hermitian post-process + output conversion shared by the STFT kernels.  `park` holds the upper half of the core's
+// outputs (park_upper_half); Z[k] for k < M/2 is the thread's own register value.  Each output value v goes to
+// out(i, s, bin, v), i = the compile-time block of bin k = tid + i*T:  s = 0: bin k,  s = 1: bin M - k,  s = 2: bin M/2
+// (thread 0, i = 0 only, where bins k and M - k are 0 and M).  V is float (dB flavours) or float2 (complex).
+template <class PL, int LAST, int KM, class Out>
+__device__ __forceinline__ void stft_values(const cx<float> (&x)[PL::E], const cx<float> *park, const float2 *rtw, int tid,
+                                            const StftParams &sp, Out &&out) {
     using R = float;
+    using V = stft_value_t<KM>;
     constexpr int M = PL::N, HALF = M / 2, PER = PL::E / 2;
     static_assert(PER * PL::T == HALF, "bins per thread");
-    float *odb = reinterpret_cast<float *>(sp.out) + frame * (M + 1);
-    float2 *ocx = reinterpret_cast<float2 *>(sp.out) + frame * (M + 1);
-    auto emit = [&](int k, cx<R> v) {                                   // exact forms (and the three special bins)
-        if constexpr (KM == STFT_K_COMPLEX) st_stream(ocx + k, make_float2(v.x, v.y));
-        else st_stream(odb + k, k < 3 ? 0.0f : stft_db(v.x, v.y, sp));  // DC and near-DC bins zeroed (:338-342)
+    auto conv = [&](int k, cx<R> v) -> V {                               // exact forms (and the three special bins)
+        if constexpr (KM == STFT_K_COMPLEX) return make_float2(v.x, v.y);
+        else return k < 3 ? 0.0f : stft_db(v.x, v.y, sp);               // DC and near-DC bins zeroed (:338-342)
     };
     static_for<PER>([&](auto I_) {
         CIDX(i, I_);
         const int k = tid + i * PL::T;
         const cx<R> z = x[slot_of_elem<PL, LAST>(i)];                   // Z[k]: this thread's own output
         if (i == 0 && k == 0) {
-            emit(0, mk<R>(z.x + z.y, 0.0f));
-            emit(M, mk<R>(z.x - z.y, 0.0f));
-            emit(HALF, RealPost<R>::middle(park[HALF], ld_tw(rtw + HALF), M));
+            out(I_, 0, 0, conv(0, mk<R>(z.x + z.y, 0.0f)));
+            out(I_, 1, M, conv(M, mk<R>(z.x - z.y, 0.0f)));
+            out(I_, 2, HALF, conv(HALF, RealPost<R>::middle(park[HALF], ld_tw(rtw + HALF), M)));
         } else {
             const cx<R> zm = park[k];
             const twd<R> w = ld_tw(rtw + k);
@@ -2280,13 +2282,13 @@ __device__ __forceinline__ void stft_post(const cx<float> (&x)[PL::E], const cx<
                 float vk = stft_db_fast(mk<R>(gr + tr, gi + ti), sp);
                 const float vm = stft_db_fast(mk<R>(gr - tr, ti - gi), sp);
                 if constexpr (i * PL::T < 3) vk = k < 3 ? 0.0f : vk;    // only the first block(s) hold bins below 3
-                st_stream(odb + k, vk);
-                st_stream(odb + (M - k), vm);
+                out(I_, 0, k, vk);
+                out(I_, 1, M - k, vm);
             } else {
                 cx<R> xk, xm;
                 RealPost<R>::pair(z, zm, w, w, xk, xm);
-                emit(k, xk);
-                emit(M - k, xm);
+                out(I_, 0, k, conv(k, xk));
+                out(I_, 1, M - k, conv(M - k, xm));
             }
         }
     });
@@ -2335,7 +2337,9 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft(const __grid_constant__
     sync_transform<PL::T, X>(xi);
     if (!active) return;
 
-    stft_post<PL, LAST, KM>(x, sm, rtw, tid, frame, sp);
+    using V = stft_value_t<KM>;
+    V *orow = reinterpret_cast<V *>(sp.out) + frame * (M + 1);
+    stft_values<PL, LAST, KM>(x, sm, rtw, tid, sp, [&](auto, int, int bin, V v) { st_stream(orow + bin, v); });
 }
 
 
@@ -2415,7 +2419,11 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_pipe(const __grid_const
         if (PL::npass() > 1) sync_transform<PL::T, X>(xi);
         park_upper_half<R, PL, LAST>(x, scratch, tid);
         sync_transform<PL::T, X>(xi);
-        if (active) stft_post<PL, LAST, KM>(x, scratch, rtw, tid, frame, sp);
+        if (active) {
+            using V = stft_value_t<KM>;
+            V *orow = reinterpret_cast<V *>(sp.out) + frame * (M + 1);
+            stft_values<PL, LAST, KM>(x, scratch, rtw, tid, sp, [&](auto, int, int bin, V v) { st_stream(orow + bin, v); });
+        }
     }
     claim_epilogue(sp.ctr);
 }
@@ -2440,53 +2448,12 @@ template <class PL, int PADQ, int X> __host__ __device__ constexpr size_t stft_w
     return ((a > b ? a : b) + 127) / 128 * 128;
 }
 
-// Hermitian post-process of one frame into REGISTER values: vk[i] = bin k = tid + i*T, vm[i] = bin M - k (thread 0:
-// vk[0] = bin 0, vm[0] = bin M, vh = bin M/2).  V is float (dB flavours) or float2 (complex).
-template <class PL, int LAST, int KM, typename V>
-__device__ __forceinline__ void stft_values(const cx<float> (&x)[PL::E], const cx<float> *park, const float2 *rtw, int tid,
-                                            const StftParams &sp, V (&vk)[PL::E / 2], V (&vm)[PL::E / 2], V &vh) {
-    using R = float;
-    constexpr int M = PL::N, HALF = M / 2, PER = PL::E / 2;
-    static_assert(PER * PL::T == HALF, "bins per thread");
-    auto conv = [&](int k, cx<R> v) -> V {                               // exact forms (and the three special bins)
-        if constexpr (KM == STFT_K_COMPLEX) return make_float2(v.x, v.y);
-        else return k < 3 ? 0.0f : stft_db(v.x, v.y, sp);               // DC and near-DC bins zeroed (:338-342)
-    };
-    static_for<PER>([&](auto I_) {
-        CIDX(i, I_);
-        const int k = tid + i * PL::T;
-        const cx<R> z = x[slot_of_elem<PL, LAST>(i)];                   // Z[k]: this thread's own output
-        if (i == 0 && k == 0) {
-            vk[0] = conv(0, mk<R>(z.x + z.y, 0.0f));
-            vm[0] = conv(M, mk<R>(z.x - z.y, 0.0f));
-            vh = conv(HALF, RealPost<R>::middle(park[HALF], ld_tw(rtw + HALF), M));
-        } else {
-            const cx<R> zm = park[k];
-            const twd<R> w = ld_tw(rtw + k);
-            if constexpr (KM == STFT_K_FAST) {
-                // 2 X[k] and 2 X[M-k]: RealPost::pair without its four multiplications by 1/2
-                const R gr = z.x + zm.x, gi = z.y - zm.y, hr = z.y + zm.y, hi = zm.x - z.x;
-                const R tr = fmaf(w.ny, hi, w.x * hr), ti = fmaf(w.y, hr, w.x * hi);
-                float a = stft_db_fast(mk<R>(gr + tr, gi + ti), sp);
-                if constexpr (i * PL::T < 3) a = k < 3 ? 0.0f : a;      // only the first block(s) hold bins below 3
-                vk[i] = a;
-                vm[i] = stft_db_fast(mk<R>(gr - tr, ti - gi), sp);
-            } else {
-                cx<R> xk, xm;
-                RealPost<R>::pair(z, zm, w, w, xk, xm);
-                vk[i] = conv(k, xk);
-                vm[i] = conv(M - k, xm);
-            }
-        }
-    });
-}
-
 template <class PL, int X, int PADQ, int MINB, int KM, bool PAD>
 __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_span(const __grid_constant__ StftParams sp) {
     static_assert(PL::valid() && PL::T * X >= 32, "needs a full issuing warp");
     extern __shared__ __align__(128) unsigned char smem_raw[];
     using R = float;
-    using V = typename std::conditional<KM == STFT_K_COMPLEX, float2, float>::type;
+    using V = stft_value_t<KM>;
     constexpr int M = PL::N, T = PL::T, E = PL::E, PER = E / 2, HALF = M / 2;
     constexpr int LAST = PL::npass() - 1;
     constexpr size_t WORK = stft_work_bytes<PL, PADQ, X>();
@@ -2585,7 +2552,10 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_span(const __grid_const
         park_upper_half<R, PL, LAST>(x, scratch, tid);
         sync_transform<T, X>(xi);
         V vk[PER], vm[PER], vh = V();
-        stft_values<PL, LAST, KM, V>(x, scratch, rtw, tid, sp, vk, vm, vh);
+        stft_values<PL, LAST, KM>(x, scratch, rtw, tid, sp, [&](auto I_, int s, int, V v) {
+            CIDX(i, I_);
+            (s == 0 ? vk[i] : s == 1 ? vm[i] : vh) = v;
+        });
         __syncthreads();                                                 // every group has read its parked half: `work` becomes the result tile
         if (geom[2 * st + 1] + xi < sp.frames) {                         // (frames of the tile's signal)
             V *orow = reinterpret_cast<V *>(reinterpret_cast<float *>(work) + out_phase(st)) + (size_t)xi * (M + 1);

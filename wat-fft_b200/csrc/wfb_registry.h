@@ -29,9 +29,19 @@ struct Variant {
     bool direct = false;   // plain global loads/stores, one launch-sized grid (no TMA pipeline, no tile counter): the zero-copy path's kernel
 };
 
-// implemented in wfb_api.cu (one launch counter / attribute cache for the whole library)
-cudaError_t launch_grid(const void *kernel, size_t smem, int threads, long ctas, const KParams &p, cudaStream_t s);
-cudaError_t launch_persistent(const void *kernel, size_t smem, int threads, long work_items, const KParams &p, cudaStream_t s);
+// Every kernel launch of the library (wfb_api.cu: one launch counter, one attribute and occupancy cache).  `params` is
+// the kernel's one parameter struct; `smem_attr` is the dynamic shared-memory limit set once per (device, kernel).  With
+// `ctr` (the struct's tile-counter field) the launch is persistent: it gets a zeroed counter and at most as many CTAs
+// as are resident on the whole GPU; otherwise the grid is `work_items` CTAs.
+cudaError_t launch(const void *kernel, size_t smem, size_t smem_attr, int threads, long work_items, void *params,
+                   unsigned long long **ctr, cudaStream_t s);
+template <class P> cudaError_t launch_grid(const void *kernel, size_t smem, int threads, long ctas, const P &p, cudaStream_t s) {
+    return launch(kernel, smem, smem, threads, ctas, (void *)&p, nullptr, s);
+}
+template <class P> cudaError_t launch_persistent(const void *kernel, size_t smem, int threads, long work_items, const P &p, cudaStream_t s) {
+    P q = p;
+    return launch(kernel, smem, smem, threads, work_items, &q, &q.ctr, s);
+}
 
 const std::vector<Variant> &variants_f32_direct();
 const std::vector<Variant> &variants_f32_x2();
@@ -194,84 +204,85 @@ template <class PL, int X, int MINB> struct RealTileLaunchers {
     }
 };
 
-// fused STFT (frame gather + window + r2c + magnitude/dB)
+// fused STFT (frame gather + window + r2c + magnitude/dB): three kernels, picked per call by stft_route (wfb_api.cu)
+enum { STFT_DIRECT = 0, STFT_SPAN = 1, STFT_PIPE = 2 };
 typedef cudaError_t (*stft_launch_fn)(const StftParams &sp, cudaStream_t s);
 struct StftVariant {
-    const char *name; int core_n; std::vector<int> radices; stft_launch_fn launch, launch_pipe, launch_span;
+    const char *name; int core_n; std::vector<int> radices;
+    stft_launch_fn launch[3];          // by route (STFT_DIRECT, STFT_SPAN, STFT_PIPE); no span kernel below N = 256
     std::vector<int> span_radices;     // stage structure of the span kernel's core plan (its own twiddle table when it differs)
+    int span_frames = 0;               // span kernel: frames per tile ...
+    size_t span_fixed_bytes = 0;       // ... and its shared memory besides the span stage
     bool span_default = false;         // measured faster than the direct kernel at hop = N/4 (profiles/): used unless WFB_STFT_SPAN says otherwise
 };
-// persistent launch whose dynamic shared memory varies from call to call (the span stages depend on hop and window)
-cudaError_t launch_persistent_dyn(const void *kernel, size_t smem, int threads, long work_items, const StftParams &sp, cudaStream_t s);
-cudaError_t launch_persistent_raw(const void *kernel, size_t smem, int threads, long work_items, void *params, cudaStream_t s);
-cudaError_t launch_grid_raw(const void *kernel, size_t smem, int threads, long ctas, void *params, cudaStream_t s);
 const std::vector<StftVariant> &variants_stft();
+constexpr size_t STFT_SPAN_SMEM_MAX = 200 * 1024;      // the span kernel's shared-memory limit; larger spans take another kernel
+// the span stage of k_stft_span: the samples of `frames` overlapping frames, in whole 128-byte lines
+inline size_t stft_span_bytes(int frames, int hop, int wsize) {
+    return ((size_t)((long)(frames - 1) * hop + wsize) * sizeof(float) + 127) / 128 * 128;
+}
+// kernel flavour: fast dB / exact dB / complex output.  The fast form drops the +1e-10 of magnitudeToDb, which lowers a
+// value by 20 log10(1 + 1e-10 / (|X| c)) dB, the most at the floor (gain - range): it runs only where that is at most
+// 1e-6 of the [0, 1] output there (floors down to about -99 dB at range 80)
+inline int stft_flavour(const StftParams &sp) {
+    if (sp.mode == STFT_MODE_COMPLEX) return STFT_K_COMPLEX;
+    const double worst = 20.0 * log10(1.0 + 1e-10 * pow(10.0, -(double)sp.db_floor / 20.0)) * (double)sp.inv_range;
+    return worst > 1e-6 ? STFT_K_EXACT : STFT_K_FAST;
+}
+// the instantiation k(KM, PAD) of an STFT kernel for a flavour; the unpadded fast-dB case (window = FFT size, the
+// spectrogram default) has its own instantiation without the per-element bound check
+template <class K> const void *stft_kernel(int flavour, bool pad, K k) {
+    using std::integral_constant;
+    switch (flavour) {
+        case STFT_K_FAST: return pad ? k(integral_constant<int, STFT_K_FAST>{}, std::true_type{}) : k(integral_constant<int, STFT_K_FAST>{}, std::false_type{});
+        case STFT_K_EXACT: return k(integral_constant<int, STFT_K_EXACT>{}, std::true_type{});
+        default: return k(integral_constant<int, STFT_K_COMPLEX>{}, std::true_type{});
+    }
+}
 template <class PL, int X, int MINB, int PQ = PADQ> struct StftLaunchers {
     static constexpr size_t smem = sizeof(cx<float>) * (size_t)padded_size<PQ>(PL::N) * X;
-    // kernel flavour: fast dB / exact dB / complex output; the unpadded fast-dB case (window = FFT size, the spectrogram
-    // default) gets its own instantiation without the per-element bound check.  The fast form drops the +1e-10 of
-    // magnitudeToDb, which lowers a value by 20 log10(1 + 1e-10 / (|X| c)) dB, the most at the floor (gain - range): it
-    // runs only where that is at most 1e-6 of the [0, 1] output there (floors down to about -99 dB at range 80)
-    static int flavour(const StftParams &sp) {
-        if (sp.mode == STFT_MODE_COMPLEX) return STFT_K_COMPLEX;
-        const double worst = 20.0 * log10(1.0 + 1e-10 * pow(10.0, -(double)sp.db_floor / 20.0)) * (double)sp.inv_range;
-        return worst > 1e-6 ? STFT_K_EXACT : STFT_K_FAST;
-    }
-    static cudaError_t launch(const StftParams &sp, cudaStream_t s) {
-        const bool pad = sp.wsize < 2 * PL::N;
-        const void *k;
-        switch (flavour(sp)) {
-            case STFT_K_FAST: k = pad ? (const void *)k_stft<PL, X, PQ, MINB, STFT_K_FAST, true> : (const void *)k_stft<PL, X, PQ, MINB, STFT_K_FAST, false>; break;
-            case STFT_K_EXACT: k = (const void *)k_stft<PL, X, PQ, MINB, STFT_K_EXACT, true>; break;
-            default: k = (const void *)k_stft<PL, X, PQ, MINB, STFT_K_COMPLEX, true>; break;
-        }
-        return launch_grid_raw(k, smem, PL::T * X, (sp.frames * sp.batch + X - 1) / X, (void *)&sp, s);
+    static cudaError_t direct(const StftParams &sp, cudaStream_t s) {
+        const void *k = stft_kernel(stft_flavour(sp), sp.wsize < 2 * PL::N, [](auto km, auto pad) {
+            return (const void *)k_stft<PL, X, PQ, MINB, decltype(km)::value, decltype(pad)::value>;
+        });
+        return launch_grid(k, smem, PL::T * X, (sp.frames * sp.batch + X - 1) / X, sp, s);
     }
     // pipelined variant: XP frames per CTA (>= one warp of threads)
     static constexpr int XP = (PL::T * X >= 128) ? X : 128 / PL::T;
     static constexpr size_t smem_pipe = 2 * real_pipe_buf_bytes<float, PL, PQ, XP, false>() + 64;
-    static cudaError_t launch_pipe(const StftParams &sp0, cudaStream_t s) {
+    static cudaError_t pipe(const StftParams &sp0, cudaStream_t s) {
         StftParams sp = sp0;
         sp.tps = (unsigned)((sp.frames + XP - 1) / XP);
         sp.tiles = (long)sp.tps * sp.batch;
         stft_tile_magic(sp);
-        const bool pad = sp.wsize < 2 * PL::N;
-        const void *k;
-        switch (flavour(sp)) {
-            case STFT_K_FAST: k = pad ? (const void *)k_stft_pipe<PL, XP, PQ, MINB, STFT_K_FAST, true> : (const void *)k_stft_pipe<PL, XP, PQ, MINB, STFT_K_FAST, false>; break;
-            case STFT_K_EXACT: k = (const void *)k_stft_pipe<PL, XP, PQ, MINB, STFT_K_EXACT, true>; break;
-            default: k = (const void *)k_stft_pipe<PL, XP, PQ, MINB, STFT_K_COMPLEX, true>; break;
-        }
-        return launch_persistent_raw(k, smem_pipe, PL::T * XP, sp.tiles, (void *)&sp, s);
+        const void *k = stft_kernel(stft_flavour(sp), sp.wsize < 2 * PL::N, [](auto km, auto pad) {
+            return (const void *)k_stft_pipe<PL, XP, PQ, MINB, decltype(km)::value, decltype(pad)::value>;
+        });
+        return launch_persistent(k, smem_pipe, PL::T * XP, sp.tiles, sp, s);
     }
-    static StftVariant make(const char *name) { return StftVariant{name, PL::N, plan_radices<PL>(), &launch, &launch_pipe, nullptr, {}}; }
+    static StftVariant make(const char *name) { return StftVariant{name, PL::N, plan_radices<PL>(), {&direct, nullptr, &pipe}}; }
 };
 
 // span-staged persistent STFT (k_stft_span): SPL = core plan (may differ from the direct kernel's: the one-exchange plans
-// the plain r2c kernels use), XS frames per tile.  Returns cudaErrorInvalidConfiguration when the tile's span does not
-// fit shared memory (very large hops): the caller falls back to the direct kernel.
-template <class PL, int X, int MINB, class SPL, int XS, int SMINB, int SPQ, bool DEFAULT> struct StftSpanLaunchers : StftLaunchers<PL, X, MINB> {
-    static cudaError_t launch_span(const StftParams &sp0, cudaStream_t s) {
+// the plain r2c kernels use), XS frames per tile.  Shared memory: the work area, the span stage, mbarriers/slots, window.
+template <class PL, int X, int MINB, class SPL, int XS, int SMINB, int SPQ, bool DEFAULT> struct StftSpanLaunchers {
+    static constexpr size_t fixed = stft_work_bytes<SPL, SPQ, XS>() + 128 + sizeof(float2) * SPL::N;
+    static cudaError_t span(const StftParams &sp0, cudaStream_t s) {
         StftParams sp = sp0;
-        const size_t span = ((size_t)((long)(XS - 1) * sp.hop + sp.wsize) * sizeof(float) + 127) / 128 * 128;
-        const size_t smem = stft_work_bytes<SPL, SPQ, XS>() + span + 128 + sizeof(float2) * SPL::N;      // + mbarriers/slots + window
-        if (smem > 200u * 1024u) return cudaErrorInvalidConfiguration;
-        sp.span_bytes = (int)span;
+        const size_t stage = stft_span_bytes(XS, sp.hop, sp.wsize);
+        sp.span_bytes = (int)stage;
         sp.tps = (unsigned)((sp.frames + XS - 1) / XS);
         sp.tiles = (long)sp.tps * sp.batch;
         stft_tile_magic(sp);
-        const bool pad = sp.wsize < 2 * SPL::N;
-        const void *k;
-        switch (StftLaunchers<PL, X, MINB>::flavour(sp)) {
-            case STFT_K_FAST: k = pad ? (const void *)k_stft_span<SPL, XS, SPQ, SMINB, STFT_K_FAST, true> : (const void *)k_stft_span<SPL, XS, SPQ, SMINB, STFT_K_FAST, false>; break;
-            case STFT_K_EXACT: k = (const void *)k_stft_span<SPL, XS, SPQ, SMINB, STFT_K_EXACT, true>; break;
-            default: k = (const void *)k_stft_span<SPL, XS, SPQ, SMINB, STFT_K_COMPLEX, true>; break;
-        }
-        return launch_persistent_dyn(k, smem, SPL::T * XS, sp.tiles, sp, s);
+        const void *k = stft_kernel(stft_flavour(sp), sp.wsize < 2 * SPL::N, [](auto km, auto pad) {
+            return (const void *)k_stft_span<SPL, XS, SPQ, SMINB, decltype(km)::value, decltype(pad)::value>;
+        });
+        return launch(k, fixed + stage, STFT_SPAN_SMEM_MAX, SPL::T * XS, sp.tiles, &sp, &sp.ctr, s);
     }
     static StftVariant make(const char *name) {
         static_assert(SPL::N == PL::N, "same core size");
-        return StftVariant{name, PL::N, plan_radices<PL>(), &StftLaunchers<PL, X, MINB>::launch, &StftLaunchers<PL, X, MINB>::launch_pipe, &launch_span, plan_radices<SPL>(), DEFAULT};
+        using D = StftLaunchers<PL, X, MINB>;
+        return StftVariant{name, PL::N, plan_radices<PL>(), {&D::direct, &span, &D::pipe}, plan_radices<SPL>(), XS, fixed, DEFAULT};
     }
 };
 
@@ -285,7 +296,7 @@ const std::vector<IstftVariant> &variants_istft();
 template <class PL, int X, int PQ, int MINB> struct IstftLaunchers {
     static constexpr size_t smem = istft_smem_bytes<PL, PQ, X>();
     static cudaError_t launch(const IstftParams &ip, long tiles, cudaStream_t s) {
-        return launch_grid_raw((const void *)k_istft<PL, X, PQ, MINB>, smem, PL::T * X, tiles, (void *)&ip, s);
+        return launch_grid((const void *)k_istft<PL, X, PQ, MINB>, smem, PL::T * X, tiles, ip, s);
     }
     static IstftVariant make(const char *name) { return IstftVariant{name, PL::N, plan_radices<PL>(), &launch, X}; }
 };
