@@ -180,20 +180,24 @@ using namespace wfb;
 // ----------------------------------------------------------------------------------------
 // plan object
 // ----------------------------------------------------------------------------------------
+// one kernel variant of a plan and its twiddle tables, built and uploaded on the variant's first launch (ensure_tables)
+struct PlanVariant {
+    const Variant *v;
+    void *d_tables = nullptr;          // the one allocation d_tw / d_rtw point into; null until the tables are uploaded
+    size_t tables_bytes = 0;
+    void *d_tw[2] = {};                // stage tables by direction (WFB_FORWARD, WFB_INVERSE)
+    void *d_rtw = nullptr;             // W_n^k of the real transforms (table format depends on the lane type)
+    std::vector<unsigned char> h_tw0[2];   // head of each stage table for KParams::tw0 (scalar-lane variants)
+};
+
 struct wfb_plan {
     int kind, precision, layout, n, device, flags;
     long batch;
     int core_n;
     size_t elem;                       // sizeof(real)
-    std::vector<const Variant *> variants;
+    std::vector<PlanVariant> variants; // every registered variant of this (precision, core size, kind), best first
     int variant;                       // forward-direction kernel variant
     int variant_inv;                   // inverse-direction kernel variant
-    void *d_tw_fwd[8], *d_tw_inv[8];   // per variant; built and uploaded on the variant's first launch (ensure_tables)
-    void *d_rtw[8];                    // per variant (table format depends on the lane type)
-    void *d_tables[8];                 // the one allocation d_tw_fwd / d_tw_inv / d_rtw of a variant point into
-    size_t tables_bytes[8];
-    bool tables_ready[8];
-    std::vector<unsigned char> h_tw0_fwd[8], h_tw0_inv[8];   // head of each table for KParams::tw0 (scalar-lane variants)
     // buffers: C2C -> plane 0 / plane 1; R2C -> time / spectrum
     void *d_buf[2];
     void *h_buf[2];
@@ -333,8 +337,8 @@ static size_t up256(size_t b) { return (b + 255) / 256 * 256; }
 
 // builds forward / inverse stage tables for one variant and uploads them
 template <typename R>
-static int upload_tables(wfb_plan *pl, int vi) {
-    const Variant &v = *pl->variants[vi];
+static int upload_tables(wfb_plan *pl, PlanVariant &pv) {
+    const Variant &v = *pv.v;
     const int m = v.core_n;
     int flavour;
     if (sizeof(R) == 8) flavour = (m == 16 || m <= 4) ? TW_EXACT : TW_F64;
@@ -361,7 +365,7 @@ static int upload_tables(wfb_plan *pl, int vi) {
             h.assign(KParams::TW0_BYTES, 0);
             memcpy(h.data(), t.data(), std::min<size_t>(t.size() * sizeof(R), KParams::TW0_BYTES));
         };
-        head(fwd, pl->h_tw0_fwd[vi]); head(inv, pl->h_tw0_inv[vi]);
+        head(fwd, pv.h_tw0[WFB_FORWARD]); head(inv, pv.h_tw0[WFB_INVERSE]);
     }
     widen(fwd); widen(inv);
     std::vector<R> packed;
@@ -379,15 +383,18 @@ static int upload_tables(wfb_plan *pl, int vi) {
     memcpy(blob.data(), fwd.data(), fwd.size() * sizeof(R));
     memcpy(blob.data() + bf, inv.data(), inv.size() * sizeof(R));
     if (!packed.empty()) memcpy(blob.data() + bf + bi, packed.data(), packed.size() * sizeof(R));
-    pl->tables_bytes[vi] = blob.size();
-    CK(dev_alloc(pl->device, blob.size(), &pl->d_tables[vi]));
+    void *d = nullptr;
+    CK(dev_alloc(pl->device, blob.size(), &d));
     // stream-ordered on the plan's stream and completed here: launches on ANY stream may follow (plan streams are
     // non-blocking, so the legacy-stream cudaMemcpy would not order against them)
-    CK(cudaMemcpyAsync(pl->d_tables[vi], blob.data(), blob.size(), cudaMemcpyHostToDevice, pl->stream));
-    CK(cudaStreamSynchronize(pl->stream));
-    pl->d_tw_fwd[vi] = pl->d_tables[vi];
-    pl->d_tw_inv[vi] = (unsigned char *)pl->d_tables[vi] + bf;
-    pl->d_rtw[vi] = packed.empty() ? nullptr : (unsigned char *)pl->d_tables[vi] + bf + bi;
+    cudaError_t e = cudaMemcpyAsync(d, blob.data(), blob.size(), cudaMemcpyHostToDevice, pl->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(pl->stream);
+    if (e != cudaSuccess) { dev_free(pl->device, d, blob.size()); return cuda_fail(e, "twiddle table upload"); }
+    pv.d_tables = d;
+    pv.tables_bytes = blob.size();
+    pv.d_tw[WFB_FORWARD] = d;
+    pv.d_tw[WFB_INVERSE] = (unsigned char *)d + bf;
+    pv.d_rtw = packed.empty() ? nullptr : (unsigned char *)d + bf + bi;
     return WFB_OK;
 }
 
@@ -395,10 +402,9 @@ static int upload_tables(wfb_plan *pl, int vi) {
 // launched get theirs: the plan's defaults at creation (this is the reference's precompute_* call), the others on
 // their first launch.
 static int ensure_tables(wfb_plan *pl, int vi) {
-    if (pl->tables_ready[vi]) return WFB_OK;
-    int rc = pl->precision == WFB_F64 ? upload_tables<double>(pl, vi) : upload_tables<float>(pl, vi);
-    if (rc == WFB_OK) pl->tables_ready[vi] = true;
-    return rc;
+    PlanVariant &pv = pl->variants[vi];
+    if (pv.d_tables) return WFB_OK;
+    return pl->precision == WFB_F64 ? upload_tables<double>(pl, pv) : upload_tables<float>(pl, pv);
 }
 
 static int ensure_device_buffers(wfb_plan *pl) {
@@ -453,7 +459,7 @@ static int plan_init(wfb_plan *pl) {
     // the zero-copy path launches the direct-load kernel (no TMA pipeline to fill, no tile counter): lowest alignment need
     pl->mapped_variant = -1;
     for (size_t i = 0; i < pl->variants.size(); i++)
-        if (pl->variants[i]->direct && pl->variants[i]->lanes == 1) { pl->mapped_variant = (int)i; break; }
+        if (pl->variants[i].v->direct && pl->variants[i].v->lanes == 1) { pl->mapped_variant = (int)i; break; }
     if (!(pl->flags & WFB_PLAN_NO_HOST_BUFFERS)) {
         // mapped + portable: the kernels can address these buffers directly (hd_buf), which is what the small-batch path does
         if (pl->kind == WFB_R2C && pl->batch == 1) {
@@ -525,20 +531,13 @@ wfb_plan *wfb_plan_create_ex(int kind, int precision, int layout, int n, long ba
     else families = {&variants_f32_tile(), &variants_f32_pipe(), &variants_f32_real_pipe(), &variants_f32_x2(), &variants_f32_direct()};
     for (const auto *fam : families)
         for (const Variant &v : *fam)
-            if (v.core_n == pl->core_n && (kind == WFB_C2C ? v.c2c != nullptr : v.r2c != nullptr)) pl->variants.push_back(&v);
+            if (v.core_n == pl->core_n && v.ops[kind == WFB_C2C ? OP_IL_FWD : OP_R2C].kernel) pl->variants.push_back({&v});
     const bool il = kind == WFB_C2C && layout == WFB_INTERLEAVED;
-    std::stable_sort(pl->variants.begin(), pl->variants.end(), [il](const Variant *a, const Variant *b) {
-        return (il ? a->priority_il : a->priority) > (il ? b->priority_il : b->priority);
+    std::stable_sort(pl->variants.begin(), pl->variants.end(), [il](const PlanVariant &a, const PlanVariant &b) {
+        return (il ? a.v->priority_il : a.v->priority) > (il ? b.v->priority_il : b.v->priority);
     });
-    if (pl->variants.size() > 8) {          // keep the 7 best plus the direct kernel (unaligned-pointer fallback, zero-copy path)
-        const Variant *fallback = pl->variants.back();
-        for (const Variant *v : pl->variants) if (v->align < fallback->align) fallback = v;
-        for (const Variant *v : pl->variants) if (v->direct && v->lanes == 1) { fallback = v; break; }
-        pl->variants.resize(7);
-        if (std::find(pl->variants.begin(), pl->variants.end(), fallback) == pl->variants.end()) pl->variants.push_back(fallback);
-    }
     for (size_t i = 0; i < pl->variants.size(); i++)
-        if (!il && pl->variants[i]->priority_inv > pl->variants[pl->variant_inv]->priority_inv) pl->variant_inv = (int)i;
+        if (!il && pl->variants[i].v->priority_inv > pl->variants[pl->variant_inv].v->priority_inv) pl->variant_inv = (int)i;
     if (pl->variants.empty()) { *err = WFB_ERR_BAD_SIZE; delete pl; return nullptr; }
     *err = plan_init(pl);
     if (*err) { wfb_plan_destroy(pl); return nullptr; }
@@ -558,7 +557,7 @@ void wfb_plan_destroy(wfb_plan *pl) {
         if (pl->pipe_done[i]) cudaEventDestroy(pl->pipe_done[i]);
     }
     if (pl->start_ev) cudaEventDestroy(pl->start_ev);
-    for (int i = 0; i < 8; i++) dev_free(pl->device, pl->d_tables[i], pl->tables_bytes[i]);
+    for (const PlanVariant &pv : pl->variants) dev_free(pl->device, pv.d_tables, pv.tables_bytes);
     for (int i = 0; i < 2; i++) dev_free(pl->device, pl->d_buf[i], pl->bytes[i]);
     if (pl->host_alias) host_free(pl->h_buf[1], pl->bytes[1]);
     else for (int i = 0; i < 2; i++) host_free(pl->h_buf[i], pl->bytes[i]);
@@ -596,7 +595,7 @@ int wfb_plan_current_variant(wfb_plan *pl, int direction) {
 }
 const char *wfb_plan_variant_name(wfb_plan *pl, int v) {
     if (!pl || v < 0 || v >= (int)pl->variants.size()) return "";
-    return pl->variants[v]->name;
+    return pl->variants[v].v->name;
 }
 size_t wfb_plan_algorithmic_bytes(wfb_plan *pl) { return pl ? payload_bytes(pl) : 0; }
 
@@ -637,32 +636,28 @@ static int launch_rows(wfb_plan *pl, int direction, const void *in0, const void 
         // direct kernels read split planes with scalar loads
         return (v->align < 16 && pl->kind == WFB_C2C && pl->layout == WFB_SPLIT) ? (int)pl->elem : v->align;
     };
-    if (bits & (uintptr_t)(need(pl->variants[vi]) - 1)) {
+    if (bits & (uintptr_t)(need(pl->variants[vi].v) - 1)) {
         int alt = -1;
         for (size_t i = 0; i < pl->variants.size() && alt < 0; i++)
-            if (!(bits & (uintptr_t)(need(pl->variants[i]) - 1))) alt = (int)i;
+            if (!(bits & (uintptr_t)(need(pl->variants[i].v) - 1))) alt = (int)i;
         if (alt < 0) return WFB_ERR_BAD_ARG;
         vi = alt;
     }
-    const Variant &v = *pl->variants[vi];
     if (int rc = ensure_tables(pl, vi)) return rc;
+    const PlanVariant &pv = pl->variants[vi];
     KParams p;
     p.in0 = in0; p.in1 = in1; p.out0 = out0; p.out1 = out1;
-    p.tw = direction == WFB_INVERSE ? pl->d_tw_inv[vi] : pl->d_tw_fwd[vi];
-    p.rtw = pl->d_rtw[vi];
+    p.tw = pv.d_tw[direction];
+    p.rtw = pv.d_rtw;
     p.batch = rows;
     p.scale = 1.0 / (double)pl->n;
     p.ctr = nullptr;
     p.done_flag = signal ? pl->hd_flag : nullptr;
     p.done_ctr = pl->d_done_ctr;
     p.done_token = pl->token;
-    const std::vector<unsigned char> &h0 = direction == WFB_INVERSE ? pl->h_tw0_inv[vi] : pl->h_tw0_fwd[vi];
-    if (!h0.empty()) memcpy(p.tw0, h0.data(), KParams::TW0_BYTES);
-    cudaError_t e;
-    if (pl->kind == WFB_C2C)
-        e = v.c2c(pl->layout == WFB_SPLIT ? IO_SPLIT : IO_INTERLEAVED, direction, p, rows, s);
-    else
-        e = direction == WFB_FORWARD ? v.r2c(0, 0, p, rows, s) : v.c2r(0, 1, p, rows, s);
+    if (!pv.h_tw0[direction].empty()) memcpy(p.tw0, pv.h_tw0[direction].data(), KParams::TW0_BYTES);
+    const int op = (pl->kind == WFB_R2C ? OP_R2C : pl->layout == WFB_SPLIT ? OP_SPLIT_FWD : OP_IL_FWD) + direction;
+    cudaError_t e = launch_op(*pv.v, op, p, rows, s);
     if (e != cudaSuccess) return cuda_fail(e, "kernel launch");
     return WFB_OK;
 }

@@ -1,32 +1,43 @@
 // wfb_registry.h -- kernel-variant registry shared by the variant translation units and the API.
 //
-// Each wfb_variants_*.cu instantiates a family of kernels and returns descriptors (Variant); the
-// API (wfb_api.cu) picks, per (precision, core size, kind), the variant with the highest priority
-// as the plan's default and keeps the others selectable (wfb_plan_set_variant) for tuning.
+// Each wfb_variants_*.cu instantiates a family of kernels and returns one descriptor (Variant) per entry.  A Variant
+// describes its launches as data: per operation (c2c split / interleaved x forward / inverse, r2c, c2r) the kernel,
+// threads per CTA, batch rows per work item and dynamic shared memory; launch_op turns one of them into a launch.  A
+// plan (wfb_api.cu) holds every registered variant of its (precision, core size, kind), ordered by priority: the first
+// is the default, the others stay selectable (wfb_plan_set_variant) for tuning and parity tests.
 #pragma once
 #include "wfb_kernels.cuh"
 
+#include <array>
 #include <vector>
 
 namespace wfb {
 
-typedef cudaError_t (*launch_fn)(int io, int dir, const KParams &p, long batch, cudaStream_t s);
+// the operations of a variant; c2c and real operations are (base + direction), direction WFB_FORWARD = 0 / WFB_INVERSE = 1
+enum { OP_SPLIT_FWD, OP_SPLIT_INV, OP_IL_FWD, OP_IL_INV, OP_R2C, OP_C2R, NOPS };
+// one operation's launch: `kernel` null = the variant does not do it; a work item is one CTA of a grid kernel or one
+// tile of a persistent one
+struct OpLaunch {
+    const void *kernel;
+    int threads;
+    int rows_per_item;
+    size_t smem;
+};
+typedef std::array<OpLaunch, NOPS> OpLaunches;
 
 struct Variant {
     const char *name;
     int core_n;        // complex points of the core transform (n for C2C, n/2 for R2C)
-    int threads;       // per CTA
-    int rows_per_cta;  // thread groups per CTA
-    size_t smem;       // dynamic shared memory per CTA
     int lanes;         // batch rows per thread group: 2 for the packed-FP32 (f32x2) kernels
     int priority;      // larger = preferred default (set from measurements, profiles/)
-    int priority_inv;  // same for the inverse direction (c2r / ifft); -1 = same as `priority`
-    int priority_il;   // same for interleaved c2c layouts; -1 = same as `priority`
+    int priority_inv;  // same for the inverse direction (c2r / ifft)
+    int priority_il;   // same for interleaved c2c layouts
     int align;         // required alignment (bytes) of every plane pointer: 16 for the TMA / float4 kernels,
                        // one complex value for the direct kernels (one scalar when the layout is split)
     std::vector<int> radices;
-    launch_fn c2c, r2c, c2r;
-    bool direct = false;   // plain global loads/stores, one launch-sized grid (no TMA pipeline, no tile counter): the zero-copy path's kernel
+    OpLaunches ops;
+    bool persistent;   // grid = resident CTAs claiming tiles from a counter (KParams::ctr)
+    bool direct;       // plain global loads/stores, one launch-sized grid (no TMA pipeline, no tile counter): the zero-copy path's kernel
 };
 
 // Every kernel launch of the library (wfb_api.cu: one launch counter, one attribute and occupancy cache).  `params` is
@@ -41,6 +52,14 @@ template <class P> cudaError_t launch_grid(const void *kernel, size_t smem, int 
 template <class P> cudaError_t launch_persistent(const void *kernel, size_t smem, int threads, long work_items, const P &p, cudaStream_t s) {
     P q = p;
     return launch(kernel, smem, smem, threads, work_items, &q, &q.ctr, s);
+}
+// operation `op` of `v` over `rows` batch rows (a persistent kernel's counter goes to p.ctr); a variant without that
+// operation gives cudaErrorInvalidDeviceFunction
+inline cudaError_t launch_op(const Variant &v, int op, KParams &p, long rows, cudaStream_t s) {
+    const OpLaunch &l = v.ops[op];
+    if (!l.kernel) return cudaErrorInvalidDeviceFunction;
+    return launch(l.kernel, l.smem, l.smem, l.threads, (rows + l.rows_per_item - 1) / l.rows_per_item, &p,
+                  v.persistent ? &p.ctr : nullptr, s);
 }
 
 const std::vector<Variant> &variants_f32_direct();
@@ -58,33 +77,37 @@ template <class PL> std::vector<int> plan_radices() {
     return r;
 }
 
+// the descriptor every family's make() returns; priority_inv and priority_il default (-1) to `priority`
+template <class PL> Variant make_variant(const char *name, int priority, int priority_inv, int priority_il, int lanes, int align,
+                                         bool persistent, const OpLaunches &ops, bool direct = false) {
+    return Variant{name, PL::N, lanes, priority, priority_inv < 0 ? priority : priority_inv, priority_il < 0 ? priority : priority_il,
+                   align, plan_radices<PL>(), ops, persistent, direct};
+}
+// the c2c records of a family: k(io, inverse) is the kernel instantiation; SPLIT = false leaves the split layout without one
+template <bool SPLIT, class K> void c2c_ops(OpLaunches &ops, int threads, int rows_per_item, size_t smem, K k) {
+    using std::integral_constant;
+    if constexpr (SPLIT) {
+        ops[OP_SPLIT_FWD] = {k(integral_constant<int, IO_SPLIT>{}, std::false_type{}), threads, rows_per_item, smem};
+        ops[OP_SPLIT_INV] = {k(integral_constant<int, IO_SPLIT>{}, std::true_type{}), threads, rows_per_item, smem};
+    }
+    ops[OP_IL_FWD] = {k(integral_constant<int, IO_INTERLEAVED>{}, std::false_type{}), threads, rows_per_item, smem};
+    ops[OP_IL_INV] = {k(integral_constant<int, IO_INTERLEAVED>{}, std::true_type{}), threads, rows_per_item, smem};
+}
+
 constexpr int PADQ = 16;   // one pad slot per 16 complex values: conflict-free for every plan (tools/bank_sim.py)
 
 // one transform (or lane pair) per thread group, X groups per CTA, direct global loads/stores
 template <typename R, class PL, int X, int MINB, bool SPLIT_IO> struct Launchers {
     static constexpr size_t smem = sizeof(cx<R>) * (size_t)padded_size<PADQ>(PL::N) * X;
     static constexpr int LANES = RT<R>::LANES;
-    static long ctas(long batch) { return ((batch + LANES - 1) / LANES + X - 1) / X; }
-    static cudaError_t c2c(int io, int dir, const KParams &p, long batch, cudaStream_t s) {
-        const void *k;
-        if (SPLIT_IO && io == IO_SPLIT) {
-            if constexpr (SPLIT_IO)
-                k = dir ? (const void *)k_c2c<R, PL, X, PADQ, IO_SPLIT, true, MINB> : (const void *)k_c2c<R, PL, X, PADQ, IO_SPLIT, false, MINB>;
-            else
-                k = nullptr;
-        } else {
-            k = dir ? (const void *)k_c2c<R, PL, X, PADQ, IO_INTERLEAVED, true, MINB> : (const void *)k_c2c<R, PL, X, PADQ, IO_INTERLEAVED, false, MINB>;
-        }
-        return launch_grid(k, smem, PL::T * X, ctas(batch), p, s);
-    }
-    static cudaError_t r2c(int, int, const KParams &p, long batch, cudaStream_t s) {
-        return launch_grid((const void *)k_r2c<R, PL, X, PADQ, MINB>, smem, PL::T * X, ctas(batch), p, s);
-    }
-    static cudaError_t c2r(int, int, const KParams &p, long batch, cudaStream_t s) {
-        return launch_grid((const void *)k_c2r<R, PL, X, PADQ, MINB>, smem, PL::T * X, ctas(batch), p, s);
-    }
     static Variant make(const char *name, int priority, int priority_inv = -1, int priority_il = -1) {
-        return Variant{name, PL::N, PL::T * X, X, smem, LANES, priority, priority_inv < 0 ? priority : priority_inv, priority_il < 0 ? priority : priority_il, 2 * (int)sizeof(typename RT<R>::scalar), plan_radices<PL>(), &c2c, &r2c, &c2r, true};
+        OpLaunches ops{};
+        c2c_ops<SPLIT_IO>(ops, PL::T * X, X * LANES, smem, [](auto io, auto inv) {
+            return (const void *)k_c2c<R, PL, X, PADQ, decltype(io)::value, decltype(inv)::value, MINB>;
+        });
+        ops[OP_R2C] = {(const void *)k_r2c<R, PL, X, PADQ, MINB>, PL::T * X, X * LANES, smem};
+        ops[OP_C2R] = {(const void *)k_c2r<R, PL, X, PADQ, MINB>, PL::T * X, X * LANES, smem};
+        return make_variant<PL>(name, priority, priority_inv, priority_il, LANES, 2 * (int)sizeof(typename RT<R>::scalar), false, ops, true);
     }
 };
 
@@ -92,34 +115,25 @@ template <typename R, class PL, int X, int MINB, bool SPLIT_IO> struct Launchers
 template <typename R, class PL, int X, int MINB, int RC = 0, int PQ = PADQ, bool TS = false, bool HT = false> struct PipeLaunchers {
     static constexpr size_t smem = 2 * pipe_buf_bytes<R, PL, PQ, X>() + 64;
     static constexpr int LANES = RT<R>::LANES;
-    static long tiles(long batch) { return (batch + X * LANES - 1) / (X * LANES); }
-    static cudaError_t c2c(int io, int dir, const KParams &p, long batch, cudaStream_t s) {
-        const void *k;
-        if (io == IO_SPLIT)
-            k = dir ? (const void *)k_c2c_pipe<R, PL, X, PQ, IO_SPLIT, true, MINB, RC, TS, HT> : (const void *)k_c2c_pipe<R, PL, X, PQ, IO_SPLIT, false, MINB, RC, TS, HT>;
-        else
-            k = dir ? (const void *)k_c2c_pipe<R, PL, X, PQ, IO_INTERLEAVED, true, MINB, RC, TS, HT> : (const void *)k_c2c_pipe<R, PL, X, PQ, IO_INTERLEAVED, false, MINB, RC, TS, HT>;
-        return launch_persistent(k, smem, PL::T * X, tiles(batch), p, s);
-    }
     static Variant make(const char *name, int priority, int priority_inv = -1, int priority_il = -1) {
-        return Variant{name, PL::N, PL::T * X, X, smem, LANES, priority, priority_inv < 0 ? priority : priority_inv, priority_il < 0 ? priority : priority_il, 16, plan_radices<PL>(), &c2c, nullptr, nullptr};
+        OpLaunches ops{};
+        c2c_ops<true>(ops, PL::T * X, X * LANES, smem, [](auto io, auto inv) {
+            return (const void *)k_c2c_pipe<R, PL, X, PQ, decltype(io)::value, decltype(inv)::value, MINB, RC, TS, HT>;
+        });
+        return make_variant<PL>(name, priority, priority_inv, priority_il, LANES, 16, true, ops);
     }
 };
 
 // register-prefetch persistent c2c (k_c2c_rpf): one transform per CTA iteration
 template <typename R, class PL, int MINB, bool TS, int PQ = PADQ> struct RegPipeLaunchers {
     static constexpr size_t smem = (TS ? 2 : 1) * pipe_buf_bytes<R, PL, PQ, 1>() + 64;
-    static cudaError_t c2c(int io, int dir, const KParams &p, long batch, cudaStream_t s) {
-        const void *k;
-        if (io == IO_SPLIT)
-            k = dir ? (const void *)k_c2c_rpf<R, PL, PQ, IO_SPLIT, true, MINB, TS> : (const void *)k_c2c_rpf<R, PL, PQ, IO_SPLIT, false, MINB, TS>;
-        else
-            k = dir ? (const void *)k_c2c_rpf<R, PL, PQ, IO_INTERLEAVED, true, MINB, TS> : (const void *)k_c2c_rpf<R, PL, PQ, IO_INTERLEAVED, false, MINB, TS>;
-        return launch_persistent(k, smem, PL::T, batch, p, s);
-    }
     static Variant make(const char *name, int priority, int priority_inv = -1, int priority_il = -1) {
+        OpLaunches ops{};
+        c2c_ops<true>(ops, PL::T, 1, smem, [](auto io, auto inv) {
+            return (const void *)k_c2c_rpf<R, PL, PQ, decltype(io)::value, decltype(inv)::value, MINB, TS>;
+        });
         // TS: bulk stores need 16-byte aligned rows; the loads are plain element loads either way
-        return Variant{name, PL::N, PL::T, 1, smem, 1, priority, priority_inv < 0 ? priority : priority_inv, priority_il < 0 ? priority : priority_il, TS ? 16 : 2 * (int)sizeof(typename RT<R>::scalar), plan_radices<PL>(), &c2c, nullptr, nullptr};
+        return make_variant<PL>(name, priority, priority_inv, priority_il, 1, TS ? 16 : 2 * (int)sizeof(typename RT<R>::scalar), true, ops);
     }
 };
 
@@ -128,79 +142,60 @@ template <typename R, class PL, int MINB, bool TS, int PQ = PADQ> struct RegPipe
 template <typename R, class PL, int X, int MINB, bool RC = false, int PQ = PADQ, bool TS = false, int XI = X, bool HT = false> struct RealPipeLaunchers {
     static constexpr size_t smem_f = 2 * real_pipe_buf_bytes<R, PL, PQ, X, false>() + 64;
     static constexpr size_t smem_i = 2 * real_pipe_buf_bytes<R, PL, PQ, XI, true>() + 64;
-    static cudaError_t r2c(int, int, const KParams &p, long batch, cudaStream_t s) {
-        return launch_persistent((const void *)k_real_pipe<R, PL, X, PQ, false, MINB, RC, TS, HT>, smem_f, PL::T * X, (batch + X - 1) / X, p, s);
-    }
-    static cudaError_t c2r(int, int, const KParams &p, long batch, cudaStream_t s) {
-        return launch_persistent((const void *)k_real_pipe<R, PL, XI, PQ, true, MINB, false, TS, HT>, smem_i, PL::T * XI, (batch + XI - 1) / XI, p, s);
-    }
     static Variant make(const char *name, int priority, int priority_inv = -1, int priority_il = -1) {
-        return Variant{name, PL::N, PL::T * X, X, smem_i > smem_f ? smem_i : smem_f, 1, priority, priority_inv < 0 ? priority : priority_inv, priority_il < 0 ? priority : priority_il, 16, plan_radices<PL>(), nullptr, &r2c, &c2r};
+        OpLaunches ops{};
+        ops[OP_R2C] = {(const void *)k_real_pipe<R, PL, X, PQ, false, MINB, RC, TS, HT>, PL::T * X, X, smem_f};
+        ops[OP_C2R] = {(const void *)k_real_pipe<R, PL, XI, PQ, true, MINB, false, TS, HT>, PL::T * XI, XI, smem_i};
+        return make_variant<PL>(name, priority, priority_inv, priority_il, 1, 16, true, ops);
     }
 };
 
 // thread-per-row tile kernels (N <= 64)
 template <class PL, int X, int MINB> struct TileLaunchers {
     static constexpr size_t smem = sizeof(float) * 2 * (size_t)(PL::N + 2) * X;
-    static cudaError_t c2c(int io, int dir, const KParams &p, long batch, cudaStream_t s) {
-        const void *k;
-        if (io == IO_SPLIT)
-            k = dir ? (const void *)k_c2c_tile<float, PL, X, IO_SPLIT, true, MINB> : (const void *)k_c2c_tile<float, PL, X, IO_SPLIT, false, MINB>;
-        else
-            k = dir ? (const void *)k_c2c_tile<float, PL, X, IO_INTERLEAVED, true, MINB> : (const void *)k_c2c_tile<float, PL, X, IO_INTERLEAVED, false, MINB>;
-        return launch_grid(k, smem, X, (batch + X - 1) / X, p, s);
-    }
     static Variant make(const char *name, int priority, int priority_inv = -1, int priority_il = -1) {
-        return Variant{name, PL::N, X, X, smem, 1, priority, priority_inv < 0 ? priority : priority_inv, priority_il < 0 ? priority : priority_il, 16, plan_radices<PL>(), &c2c, nullptr, nullptr};
+        OpLaunches ops{};
+        c2c_ops<true>(ops, X, X, smem, [](auto io, auto inv) {
+            return (const void *)k_c2c_tile<float, PL, X, decltype(io)::value, decltype(inv)::value, MINB>;
+        });
+        return make_variant<PL>(name, priority, priority_inv, priority_il, 1, 16, false, ops);
     }
 };
 
-// persistent, fully TMA-fed thread-per-row c2c (N <= 64)
+// persistent, fully TMA-fed thread-per-row c2c (N <= 64); the f64 kernels are interleaved only
 template <class PL, int X, int MINB, typename R = float> struct TilePipeLaunchers {
     static constexpr bool F64 = sizeof(R) == 8;
     static constexpr size_t smem_i = 2 * tpipe_buf_bytes<R, PL, X, IO_INTERLEAVED>() + 64;
     static constexpr size_t smem_s = F64 ? 0 : 2 * tpipe_buf_bytes<float, PL, X, IO_SPLIT>() + 64;
     static constexpr size_t smem = smem_s > smem_i ? smem_s : smem_i;
-    static cudaError_t c2c(int io, int dir, const KParams &p, long batch, cudaStream_t s) {
-        const void *k;
-        if (io == IO_SPLIT) {
-            if constexpr (F64) return cudaErrorInvalidDeviceFunction;      // the f64 modules are interleaved only
-            else k = dir ? (const void *)k_c2c_tpipe<float, PL, X, IO_SPLIT, true, MINB> : (const void *)k_c2c_tpipe<float, PL, X, IO_SPLIT, false, MINB>;
-        } else {
-            k = dir ? (const void *)k_c2c_tpipe<R, PL, X, IO_INTERLEAVED, true, MINB> : (const void *)k_c2c_tpipe<R, PL, X, IO_INTERLEAVED, false, MINB>;
-        }
-        return launch_persistent(k, smem, X, (batch + X - 1) / X, p, s);
-    }
     static Variant make(const char *name, int priority, int priority_inv = -1, int priority_il = -1) {
-        return Variant{name, PL::N, X, X, smem, 1, priority, priority_inv < 0 ? priority : priority_inv, priority_il < 0 ? priority : priority_il, 16, plan_radices<PL>(), &c2c, nullptr, nullptr};
+        OpLaunches ops{};
+        c2c_ops<!F64>(ops, X, X, smem, [](auto io, auto inv) {
+            return (const void *)k_c2c_tpipe<R, PL, X, decltype(io)::value, decltype(inv)::value, MINB>;
+        });
+        return make_variant<PL>(name, priority, priority_inv, priority_il, 1, 16, true, ops);
     }
 };
 
 // persistent, fully TMA-fed thread-per-row r2c / c2r (N = 64, 128)
 template <class PL, int X, int MINB, typename R = float> struct RealTilePipeLaunchers {
     static constexpr size_t smem = 2 * rtpipe_buf_bytes<R, PL, X>() + 64;
-    static cudaError_t r2c(int, int, const KParams &p, long batch, cudaStream_t s) {
-        return launch_persistent((const void *)k_real_tpipe<R, PL, X, false, MINB>, smem, X, (batch + X - 1) / X, p, s);
-    }
-    static cudaError_t c2r(int, int, const KParams &p, long batch, cudaStream_t s) {
-        return launch_persistent((const void *)k_real_tpipe<R, PL, X, true, MINB>, smem, X, (batch + X - 1) / X, p, s);
-    }
     static Variant make(const char *name, int priority, int priority_inv = -1, int priority_il = -1) {
-        return Variant{name, PL::N, X, X, smem, 1, priority, priority_inv < 0 ? priority : priority_inv, priority_il < 0 ? priority : priority_il, 16, plan_radices<PL>(), nullptr, &r2c, &c2r};
+        OpLaunches ops{};
+        ops[OP_R2C] = {(const void *)k_real_tpipe<R, PL, X, false, MINB>, X, X, smem};
+        ops[OP_C2R] = {(const void *)k_real_tpipe<R, PL, X, true, MINB>, X, X, smem};
+        return make_variant<PL>(name, priority, priority_inv, priority_il, 1, 16, true, ops);
     }
 };
 
 // thread-per-row tile kernels for the real transforms (core M <= 64)
 template <class PL, int X, int MINB> struct RealTileLaunchers {
     static constexpr size_t smem = sizeof(float) * (size_t)(2 * PL::N + 4) * X;
-    static cudaError_t r2c(int, int, const KParams &p, long batch, cudaStream_t s) {
-        return launch_grid((const void *)k_r2c_tile<PL, X, MINB>, smem, X, (batch + X - 1) / X, p, s);
-    }
-    static cudaError_t c2r(int, int, const KParams &p, long batch, cudaStream_t s) {
-        return launch_grid((const void *)k_c2r_tile<PL, X, MINB>, smem, X, (batch + X - 1) / X, p, s);
-    }
     static Variant make(const char *name, int priority, int priority_inv = -1, int priority_il = -1) {
-        return Variant{name, PL::N, X, X, smem, 1, priority, priority_inv < 0 ? priority : priority_inv, priority_il < 0 ? priority : priority_il, 16, plan_radices<PL>(), nullptr, &r2c, &c2r};
+        OpLaunches ops{};
+        ops[OP_R2C] = {(const void *)k_r2c_tile<PL, X, MINB>, X, X, smem};
+        ops[OP_C2R] = {(const void *)k_c2r_tile<PL, X, MINB>, X, X, smem};
+        return make_variant<PL>(name, priority, priority_inv, priority_il, 1, 16, false, ops);
     }
 };
 
