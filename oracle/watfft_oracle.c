@@ -447,7 +447,11 @@ WFO_API void wfo_rfft_f64(int n, double *data) {
 /* f64 c2r: the reference has NO implementation (fft_real_combined.wat exports only
  * precompute_rfft_twiddles and rfft; index.js:145-147 calls a missing export).
  * PARITY UNPINNED: defined here as the exact algebraic inverse of wfo_rfft_f64's
- * formulas and gated against the f64 DFT only. */
+ * formulas, in the order of the f32 pre-process ($irfft_preprocess_split :1656-1748),
+ * and gated against the f64 DFT.  The k = M/2 bin pairs with itself: the forward form
+ * is stored first and the mirrored one survives, like wfo_irfft_split_f32 and every
+ * c2r kernel.  (The two differ by 2*wr[M/2]*Im X[M/2], and the Taylor table's
+ * wr[M/2] = cos(pi/2) is ~1e-11, not 0.) */
 WFO_API void wfo_irfft_f64(int n, const double *spec, double *x) {
     int m = n / 2;
     double *re = (double *)malloc(sizeof(double) * 4 * (size_t)(m + 1)), *im = re + (m + 1);
@@ -462,8 +466,8 @@ WFO_API void wfo_irfft_f64(int n, const double *spec, double *x) {
         double gr = ar + br, gi = ai - bi, ur = ar - br, ui = ai + bi;
         double hr = wr[k] * ur + wi[k] * ui;
         double hi = wr[k] * ui - wi[k] * ur;
-        re[m - k] = sc * (gr + hi); im[m - k] = sc * (hr - gi);
         re[k] = sc * (gr - hi); im[k] = sc * (gi + hr);
+        re[m - k] = sc * (gr + hi); im[m - k] = sc * (hr - gi);
     }
     c2c_f64_core(m, re, im, 1);
     for (int j = 0; j < m; j++) { x[2 * j] = re[j]; x[2 * j + 1] = im[j]; }

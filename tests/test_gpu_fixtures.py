@@ -390,3 +390,73 @@ def test_exec_device_misaligned_pointers_fall_back(wf, oracle):
         assert rel_err(np.r_[gr[r], gi[r]], np.r_[er, ei], np.r_[re[r], im[r]]) <= f32_bound(n)
     assert float(o_re[0]) == 0.0 and float(o_re[pad + batch * n]) == 0.0     # nothing written outside
     plan.destroy()
+
+
+MISALIGNED = [(kind, n) for kind, sizes in (("c2c f32 split", (16, 512, 8192)), ("c2c f32 interleaved", (16, 512, 8192)),
+                                             ("c2c f64", (16, 512, 8192)), ("r2c f32", (16, 1024, 16384)),
+                                             ("r2c f64", (16, 1024, 16384))) for n in sizes]
+
+
+@pytest.mark.parametrize("kind,n", MISALIGNED)
+def test_exec_device_misaligned_pointers_per_kind(wf, oracle, kind, n):
+    """Caller pointers off the 16-byte grid by one scalar or one complex value, in every kind and both directions.  Split
+    c2c is served one scalar off (the direct kernel reads scalars); interleaved c2c and r2c / c2r are served one complex
+    value off (8 bytes in f32: the direct kernel; 16 bytes in f64: every variant) and refuse one scalar off with
+    WFB_ERR_BAD_ARG, leaving the output untouched.  A served call matches the oracle on every row and writes nothing
+    outside its output rows."""
+    import torch
+    C = wf._cabi
+    dev = torch.device("cuda:0")
+    f64, real, split = "f64" in kind, kind.startswith("r2c"), "split" in kind
+    dt, tdt, elem = (np.float64, torch.float64, 8) if f64 else (np.float32, torch.float32, 4)
+    batch, guard = 33, 4096                                   # guard: scalars before and after, a multiple of 16 bytes
+    plan = wf.Plan(C.R2C if real else C.C2C, C.F64 if f64 else C.F32, C.SPLIT if split else C.INTERLEAVED, n, batch, 0,
+                   C.PLAN_NO_HOST_BUFFERS | C.PLAN_NO_DEVICE_BUFFERS)
+    rng = np.random.default_rng(n + 31)
+    for direction in (C.FORWARD, C.INVERSE):
+        inv = direction == C.INVERSE
+        li, lo = ((n + 2, n) if inv else (n, n + 2)) if real else ((n, n) if split else (2 * n, 2 * n))
+        x = [rng.uniform(-1, 1, (batch, li)).astype(dt) for _ in range(2 if split else 1)]
+        for r in range(batch):
+            if split:
+                want = np.concatenate(oracle.fft_split_f32(x[0][r], x[1][r], inv))
+            elif not real:
+                want = (oracle.fft_f64 if f64 else oracle.fft_interleaved_f32)(x[0][r], inv)
+            elif inv:
+                want = (oracle.irfft_f64 if f64 else oracle.irfft_split_f32)(x[0][r])
+            else:
+                want = (oracle.rfft_f64 if f64 else oracle.rfft_split_f32)(x[0][r])
+            if r == 0:
+                ref = np.empty((batch, want.size))
+            ref[r] = want
+        for off, served in ((1, True),) if split else ((1, False), (2, True)):     # scalars off the 16-byte grid
+            ins, outs = [], []
+            for p in x:
+                t = torch.zeros(2 * guard + batch * li, dtype=tdt, device=dev)
+                t[guard + off:guard + off + batch * li] = torch.from_numpy(p.ravel()).to(dev)
+                o = torch.empty(2 * guard + batch * lo, dtype=tdt, device=dev)
+                o.view(torch.int32).fill_(0x5AA5C33C)
+                o[guard + off:guard + off + batch * lo] = float("nan")
+                ins.append(t)
+                outs.append(o)
+            before = [o.clone() for o in outs]
+            at = lambda ts: tuple(t.data_ptr() + (guard + off) * elem for t in ts) + (None,) * (2 - len(ts))
+            torch.cuda.synchronize()      # torch filled the buffers on ITS stream; the plan's stream is non-blocking
+            tag = (kind, n, "inverse" if inv else "forward", f"{off * elem} bytes off")
+            if not served:
+                with pytest.raises(wf.WatFFTError) as e:
+                    plan.exec_device(direction, at(ins), at(outs))
+                assert e.value.code == C.ERR_BAD_ARG, tag
+                plan.sync()
+                assert all(torch.equal(o.view(torch.int32), b.view(torch.int32)) for o, b in zip(outs, before)), tag
+                continue
+            plan.exec_device(direction, at(ins), at(outs))
+            plan.sync()
+            for o, b in zip(outs, before):
+                assert torch.equal(o[:guard + off].view(torch.int32), b[:guard + off].view(torch.int32)), (tag, "wrote before")
+                assert torch.equal(o[guard + off + batch * lo:].view(torch.int32), b[guard + off + batch * lo:].view(torch.int32)), (tag, "wrote after")
+            got = np.concatenate([o[guard + off:guard + off + batch * lo].cpu().numpy().reshape(batch, lo) for o in outs], axis=1)
+            xin = np.concatenate(x, axis=1)
+            for r in range(batch):
+                assert rel_err(got[r], ref[r], xin[r]) <= (f64_bound(n) if f64 else f32_bound(n)), (tag, r)
+    plan.destroy()

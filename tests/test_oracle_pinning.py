@@ -126,3 +126,21 @@ def test_trig_accuracy_levels(oracle):
         re, im = oracle.twiddles("split", n)
         err = np.max(np.abs((re.astype(np.float64) + 1j * im) - np.exp(-2j * np.pi * k / n)))
         assert err < 1.2e-6
+
+
+@pytest.mark.parametrize("n", [1 << k for k in range(3, 15)])
+def test_oracle_irfft_f64(oracle, n):
+    """f64 c2r has no reference module (the restatement defines it), so it is pinned to the truth: numpy's inverse real DFT
+    of an exact Hermitian half spectrum, and the inverse of the oracle's own rfft_f64, both at the level of the reference's
+    Taylor-series f64 twiddles (~6.5e-11 each); the imaginary parts of DC and Nyquist are ignored, bit for bit."""
+    rng = np.random.default_rng(n + 99)
+    x = rng.uniform(-1, 1, n)
+    s = np.fft.rfft(x)
+    il = np.empty(n + 2)
+    il[0::2], il[1::2] = s.real, s.imag
+    y = oracle.irfft_f64(il)
+    assert np.max(np.abs(y - np.fft.irfft(s, n))) < 2e-9
+    assert np.max(np.abs(oracle.irfft_f64(oracle.rfft_f64(x)) - x)) < 2e-9
+    g = il.copy()
+    g[1], g[n + 1] = 123.0, -77.0
+    assert np.array_equal(oracle.irfft_f64(g), y)
