@@ -217,10 +217,27 @@ WFB_API wfb_stft *wfb_stft_create(int fft_size, int zero_padding, int hop, int w
                                   int mode, float gain_db, float range_db, int device, int flags, int *err);
 WFB_API wfb_stft *wfb_stft_create_ex(int fft_size, int zero_padding, int hop, int window_type, long num_samples,
                                      long batch, int mode, float gain_db, float range_db, int device, int flags, int *err);
+/* Filterbank spectrogram (mel and the like; an extension: the reference has none), still ONE kernel launch:
+ *   out[b][f][m] = L( sum_k F[m][k] * |X_bf[k]|^power ),
+ * X_bf the raw (unnormalised) spectrum of frame f of signal b exactly as WFB_STFT_COMPLEX writes it, F a dense host
+ * matrix float [num_filters][fft_size/2+1] (copied at creation; stored band-sparse on the device: each filter from its
+ * first to its last non-zero bin), L(v) = v when log_scale == 0, else log_scale * log2(max(v + log_offset, log_floor))
+ * (log_scale = ln 2 gives ln, log10(2) log10, 10 log10(2) dB of a power).  No bin is zeroed.
+ * Output float [batch][frames][num_filters].  Each filter is one f32 FMA chain over its band in increasing bin order, so
+ * results are bitwise repeatable and a batch row is bit-for-bit the single-signal result on the same kernel.
+ * Geometry (fft_size, zero_padding, hop, window_type, num_samples, batch) as wfb_stft_create_ex, with num_filters floats
+ * per output row in the overflow checks.  WFB_ERR_BAD_ARG also when num_filters is not in [1, fft_size/2+1], filters is
+ * NULL or holds a non-finite value, power is not 1 or 2, log_scale is not finite, or log_scale != 0 and log_floor is not
+ * a finite value > 0 or log_offset not a finite value >= 0.  The exec, buffer and size calls work unchanged;
+ * wfb_stft_exec_inverse* returns WFB_ERR_UNSUPPORTED. */
+WFB_API wfb_stft *wfb_stft_create_filterbank(int fft_size, int zero_padding, int hop, int window_type, long num_samples,
+                                             long batch, int num_filters, const float *filters, int power, float log_scale,
+                                             float log_offset, float log_floor, int device, int flags, int *err);
 WFB_API void wfb_stft_destroy(wfb_stft *st);
 WFB_API long wfb_stft_frames(wfb_stft *st);             /* per signal */
 WFB_API long wfb_stft_batch(wfb_stft *st);
 WFB_API int wfb_stft_bins(wfb_stft *st);
+WFB_API int wfb_stft_filters(wfb_stft *st);             /* num_filters; 0 for a dB or complex handle */
 WFB_API void *wfb_stft_host_samples(wfb_stft *st);      /* pinned, batch x num_samples floats */
 WFB_API void *wfb_stft_host_output(wfb_stft *st);       /* pinned, wfb_stft_output_bytes() */
 WFB_API size_t wfb_stft_output_bytes(wfb_stft *st);

@@ -7,7 +7,7 @@ the build image has no JS runtime, and binds the very same C ABI (include/watfft
 """
 from . import _cabi
 from ._cabi import WatFFTError, build
-from .stft import Spectrogram, generateSpectrogram, inverseSpectrogram
+from .stft import Spectrogram, generateSpectrogram, inverseSpectrogram, mel_filterbank, melSpectrogram
 from .contexts import (
     createFFT, createFFTf32, createRFFT, createRFFTf32,
     createFFTf32Split, createRFFTf32Split, SplitExportsFacade, ModuleExports, HostMemory, Plan,
@@ -18,5 +18,5 @@ __all__ = [
     "createFFT", "createFFTf32", "createRFFT", "createRFFTf32",
     "createFFTf32Split", "createRFFTf32Split", "SplitExportsFacade", "ModuleExports", "HostMemory", "Plan",
     "createFFTInstance", "createFFTf32Instance", "createRFFTInstance", "createRFFTf32Instance", "createFFTf32SplitInstance",
-    "Spectrogram", "generateSpectrogram", "inverseSpectrogram", "WatFFTError", "build", "_cabi",
+    "Spectrogram", "generateSpectrogram", "inverseSpectrogram", "mel_filterbank", "melSpectrogram", "WatFFTError", "build", "_cabi",
 ]

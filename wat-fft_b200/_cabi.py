@@ -71,10 +71,14 @@ SYMBOLS = {
                                            ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_int)]),
     "wfb_stft_create_ex": (ctypes.c_void_p, [ctypes.c_int] * 4 + [ctypes.c_long, ctypes.c_long, ctypes.c_int, ctypes.c_float,
                                               ctypes.c_float, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_int)]),
+    "wfb_stft_create_filterbank": (ctypes.c_void_p, [ctypes.c_int] * 4 + [ctypes.c_long, ctypes.c_long, ctypes.c_int,
+                                                      ctypes.POINTER(ctypes.c_float), ctypes.c_int] + [ctypes.c_float] * 3
+                                   + [ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_int)]),
     "wfb_stft_destroy": (None, [ctypes.c_void_p]),
     "wfb_stft_frames": (ctypes.c_long, [ctypes.c_void_p]),
     "wfb_stft_batch": (ctypes.c_long, [ctypes.c_void_p]),
     "wfb_stft_bins": (ctypes.c_int, [ctypes.c_void_p]),
+    "wfb_stft_filters": (ctypes.c_int, [ctypes.c_void_p]),
     "wfb_stft_host_samples": (ctypes.c_void_p, [ctypes.c_void_p]),
     "wfb_stft_host_output": (ctypes.c_void_p, [ctypes.c_void_p]),
     "wfb_stft_output_bytes": (ctypes.c_size_t, [ctypes.c_void_p]),
@@ -86,6 +90,7 @@ SYMBOLS = {
 }
 WINDOWS = {"hann": 0, "hamming": 1, "blackman": 2, "blackmanHarris": 3, "rectangular": 4}
 STFT_DB, STFT_COMPLEX = 0, 1
+STFT_FILTERBANK = 2      # the mode of a wfb_stft_create_filterbank handle (wfb_stft_create_ex rejects it)
 
 _lib = None
 

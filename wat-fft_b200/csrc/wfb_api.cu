@@ -1002,6 +1002,13 @@ struct wfb_stft {
     void *h_samples, *h_out;
     size_t in_bytes, out_bytes;        // whole batch
     float db_floor, inv_range;
+    // filterbank handles (mode STFT_MODE_FILTERBANK): the filters' bands {first bin, bins, weight offset, 0} and packed
+    // weights (host copies; device copies in d_tables), the power and L
+    int num_filters, power;
+    float log_scale, log_offset, log_floor;
+    std::vector<int> fb_band;
+    std::vector<float> fb_w;
+    void *d_fb_band, *d_fb_w;
     cudaStream_t stream;
     // inverse (wfb_stft_exec_inverse*): built on the first inverse call, so a forward-only handle never pays for it
     const IstftVariant *inv_variant;
@@ -1037,12 +1044,16 @@ static int stft_init(wfb_stft *st) {
     base_twiddles<float>(TW_F32_SPLIT, n, m + 1, rre, rim);
     for (int k = 0; k <= m; k++) { packed.push_back(rre[k]); packed.push_back(rim[k]); }
     for (int i = 0; i < st->wsize; i++) win[i] = (float)window_value(st->window, i, st->wsize);
-    // one allocation and one copy: [forward | span forward | W_n^k | window], each 256-byte aligned
-    const std::vector<float> *sec[4] = {&fwd, &fwd_span, &packed, &win};
-    size_t off[5] = {0};
-    for (int i = 0; i < 4; i++) off[i + 1] = off[i] + up256(sec[i]->size() * sizeof(float));
-    std::vector<unsigned char> blob(off[4], 0);
-    for (int i = 0; i < 4; i++) if (!sec[i]->empty()) memcpy(blob.data() + off[i], sec[i]->data(), sec[i]->size() * sizeof(float));
+    // one allocation and one copy: [forward | span forward | W_n^k | window | filter bands | filter weights], each
+    // 256-byte aligned (the last two are empty but for filterbank handles)
+    const std::pair<const void *, size_t> sec[6] = {
+        {fwd.data(), fwd.size() * sizeof(float)}, {fwd_span.data(), fwd_span.size() * sizeof(float)},
+        {packed.data(), packed.size() * sizeof(float)}, {win.data(), win.size() * sizeof(float)},
+        {st->fb_band.data(), st->fb_band.size() * sizeof(int)}, {st->fb_w.data(), st->fb_w.size() * sizeof(float)}};
+    size_t off[7] = {0};
+    for (int i = 0; i < 6; i++) off[i + 1] = off[i] + up256(sec[i].second);
+    std::vector<unsigned char> blob(off[6], 0);
+    for (int i = 0; i < 6; i++) if (sec[i].second) memcpy(blob.data() + off[i], sec[i].first, sec[i].second);
     CK(cudaMalloc(&st->d_tables, blob.size()));
     // stream-ordered on the handle's stream and completed here: launches on ANY stream may follow
     CK(cudaMemcpyAsync(st->d_tables, blob.data(), blob.size(), cudaMemcpyHostToDevice, st->stream));
@@ -1052,6 +1063,8 @@ static int stft_init(wfb_stft *st) {
     st->d_tw_span = fwd_span.empty() ? nullptr : d + off[1];
     st->d_rtw = d + off[2];
     st->d_window = d + off[3];
+    st->d_fb_band = st->fb_band.empty() ? nullptr : d + off[4];
+    st->d_fb_w = st->fb_w.empty() ? nullptr : d + off[5];
     if (!(st->flags & WFB_PLAN_NO_DEVICE_BUFFERS)) {
         if (cudaMalloc(&st->d_samples, st->in_bytes) != cudaSuccess) { cudaGetLastError(); return WFB_ERR_ALLOC; }
         if (cudaMalloc(&st->d_out, st->out_bytes) != cudaSuccess) { cudaGetLastError(); return WFB_ERR_ALLOC; }
@@ -1090,19 +1103,19 @@ wfb_stft *wfb_stft_create(int fft_size, int zero_padding, int hop, int window_ty
     return wfb_stft_create_ex(fft_size, zero_padding, hop, window_type, num_samples, 1, mode, gain_db, range_db, device, flags, err);
 }
 
-wfb_stft *wfb_stft_create_ex(int fft_size, int zero_padding, int hop, int window_type, long num_samples, long batch, int mode,
-                             float gain_db, float range_db, int device, int flags, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    if (!is_pow2(fft_size) || fft_size < 64 || fft_size > 8192) { *err = WFB_ERR_BAD_SIZE; return nullptr; }
+}  // extern "C"
+
+// The geometry checks and the handle of every mode, before its tables are built: the caller has checked fft_size and its
+// mode's own arguments.  row_floats: output floats per frame.
+static wfb_stft *stft_new(int fft_size, int zero_padding, int hop, int window_type, long num_samples, long batch, int mode,
+                          size_t row_floats, int device, int flags, int *err) {
     if (zero_padding < 1 || !is_pow2(zero_padding) || zero_padding > fft_size / 2 || hop < 1 ||
-        window_type < 0 || window_type > WFB_WINDOW_RECTANGULAR || (mode != WFB_STFT_DB && mode != WFB_STFT_COMPLEX) ||
-        !(range_db > 0.0f)) { *err = WFB_ERR_BAD_ARG; return nullptr; }
+        window_type < 0 || window_type > WFB_WINDOW_RECTANGULAR) { *err = WFB_ERR_BAD_ARG; return nullptr; }
     const int wsize = fft_size / zero_padding;
     if (num_samples < wsize) { *err = WFB_ERR_BAD_ARG; return nullptr; }      // "Audio too short" (spectrogram.js:299-301)
-    // the whole batch's input and output must be addressable: batch * num_samples floats, batch * frames * bins values
+    // the whole batch's input and output must be addressable: batch * num_samples floats, batch * frames * row values
     const size_t frames = (size_t)((num_samples - wsize) / hop + 1);
-    const size_t row_bytes = (size_t)(fft_size / 2 + 1) * sizeof(float) * (mode == WFB_STFT_COMPLEX ? 2 : 1);
+    const size_t row_bytes = row_floats * sizeof(float);
     size_t in_bytes, out_bytes;
     if (batch < 1 || __builtin_mul_overflow((size_t)num_samples, sizeof(float), &in_bytes) ||
         __builtin_mul_overflow(in_bytes, (size_t)batch, &in_bytes) || __builtin_mul_overflow(frames, row_bytes, &out_bytes) ||
@@ -1116,16 +1129,68 @@ wfb_stft *wfb_stft_create_ex(int fft_size, int zero_padding, int hop, int window
     st->num_samples = num_samples;
     st->frames = (long)frames;
     st->batch = batch;
-    st->db_floor = gain_db - range_db;
-    st->inv_range = 1.0f / range_db;
     st->in_bytes = in_bytes;
     st->out_bytes = out_bytes;
     for (const StftVariant &v : variants_stft()) if (v.core_n == fft_size / 2) st->variant = &v;
     if (!st->variant) { *err = WFB_ERR_BAD_SIZE; delete st; return nullptr; }
     for (const IstftVariant &v : variants_istft()) if (v.core_n == fft_size / 2) st->inv_variant = &v;
+    return st;
+}
+
+static wfb_stft *stft_ready(wfb_stft *st, int *err) {
     *err = stft_init(st);
     if (*err) { wfb_stft_destroy(st); return nullptr; }
     return st;
+}
+
+extern "C" {
+
+wfb_stft *wfb_stft_create_ex(int fft_size, int zero_padding, int hop, int window_type, long num_samples, long batch, int mode,
+                             float gain_db, float range_db, int device, int flags, int *err) {
+    int dummy;
+    if (!err) err = &dummy;
+    if (!is_pow2(fft_size) || fft_size < 64 || fft_size > 8192) { *err = WFB_ERR_BAD_SIZE; return nullptr; }
+    if ((mode != WFB_STFT_DB && mode != WFB_STFT_COMPLEX) || !(range_db > 0.0f)) { *err = WFB_ERR_BAD_ARG; return nullptr; }
+    const size_t row_floats = (size_t)(fft_size / 2 + 1) * (mode == WFB_STFT_COMPLEX ? 2 : 1);
+    wfb_stft *st = stft_new(fft_size, zero_padding, hop, window_type, num_samples, batch, mode, row_floats, device, flags, err);
+    if (!st) return nullptr;
+    st->db_floor = gain_db - range_db;
+    st->inv_range = 1.0f / range_db;
+    return stft_ready(st, err);
+}
+
+wfb_stft *wfb_stft_create_filterbank(int fft_size, int zero_padding, int hop, int window_type, long num_samples, long batch,
+                                     int num_filters, const float *filters, int power, float log_scale, float log_offset,
+                                     float log_floor, int device, int flags, int *err) {
+    int dummy;
+    if (!err) err = &dummy;
+    if (!is_pow2(fft_size) || fft_size < 64 || fft_size > 8192) { *err = WFB_ERR_BAD_SIZE; return nullptr; }
+    const int bins = fft_size / 2 + 1;
+    const bool log_ok = std::isfinite(log_scale) &&
+        (log_scale == 0.0f || (std::isfinite(log_floor) && log_floor > 0.0f && std::isfinite(log_offset) && log_offset >= 0.0f));
+    if (num_filters < 1 || num_filters > bins || !filters || (power != 1 && power != 2) || !log_ok) {
+        *err = WFB_ERR_BAD_ARG;
+        return nullptr;
+    }
+    for (size_t i = 0; i < (size_t)num_filters * bins; i++)
+        if (!std::isfinite(filters[i])) { *err = WFB_ERR_BAD_ARG; return nullptr; }
+    wfb_stft *st = stft_new(fft_size, zero_padding, hop, window_type, num_samples, batch, STFT_MODE_FILTERBANK,
+                            (size_t)num_filters, device, flags, err);
+    if (!st) return nullptr;
+    st->num_filters = num_filters;
+    st->power = power;
+    st->log_scale = log_scale; st->log_offset = log_offset; st->log_floor = log_floor;
+    // each filter's band runs from its first to its last non-zero weight (zeros inside it stay); all zero: 0 bins
+    for (int m = 0; m < num_filters; m++) {
+        const float *f = filters + (size_t)m * bins;
+        int lo = 0, hi = bins - 1;
+        while (lo < bins && f[lo] == 0.0f) lo++;
+        while (hi >= lo && f[hi] == 0.0f) hi--;
+        const int count = lo < bins ? hi - lo + 1 : 0;
+        st->fb_band.insert(st->fb_band.end(), {count ? lo : 0, count, (int)st->fb_w.size(), 0});
+        st->fb_w.insert(st->fb_w.end(), f + lo, f + lo + count);
+    }
+    return stft_ready(st, err);
 }
 
 void wfb_stft_destroy(wfb_stft *st) {
@@ -1143,6 +1208,7 @@ void wfb_stft_destroy(wfb_stft *st) {
 long wfb_stft_frames(wfb_stft *st) { return st ? st->frames : 0; }
 long wfb_stft_batch(wfb_stft *st) { return st ? st->batch : 0; }
 int wfb_stft_bins(wfb_stft *st) { return st ? st->fft_size / 2 + 1 : 0; }
+int wfb_stft_filters(wfb_stft *st) { return st ? st->num_filters : 0; }
 void *wfb_stft_host_samples(wfb_stft *st) { return st ? st->h_samples : nullptr; }
 void *wfb_stft_host_output(wfb_stft *st) { return st ? st->h_out : nullptr; }
 size_t wfb_stft_output_bytes(wfb_stft *st) { return st ? st->out_bytes : 0; }
@@ -1159,6 +1225,9 @@ int wfb_stft_exec_device(wfb_stft *st, const float *d_samples, void *d_out, void
     sp.ctr = nullptr;
     sp.span_bytes = 0;
     sp.tiles = 0; sp.tps = sp.tps_magic = 0; sp.tps_shift = 0;      // (set by the persistent kernels' launchers)
+    sp.fb_band = (const int4 *)st->d_fb_band; sp.fb_w = (const float *)st->d_fb_w;
+    sp.fb_n = st->num_filters; sp.fb_power = st->power;
+    sp.fb_scale = st->log_scale; sp.fb_offset = st->log_offset; sp.fb_floor = st->log_floor;
     // a caller's pointer may be any float address (scalar loads then); the rows of a batch keep the base's alignment only
     // when num_samples is a multiple of 2 (8 bytes) or 4 (16 bytes, the bulk-copy kernels: stft_route)
     sp.aligned8 = ((uintptr_t)d_samples % 8) == 0 && (st->batch == 1 || st->num_samples % 2 == 0);

@@ -2212,8 +2212,13 @@ struct StftParams {
     float lg_a, lg_b;          // fast dB path: value = lg_a * log2(|2 X|^2) + lg_b (host-folded constants)
     int aligned8;              // every signal's `samples` row is 8-byte aligned: even hops may use 64-bit loads
     int span_bytes;            // span kernel: shared-memory bytes of one span stage (multiple of 128)
+    // MODE_FILTERBANK: out is float [batch][frames][fb_n], out = L(sum_k F[m][k] |X[k]|^fb_power), F band-sparse:
+    const int4 *fb_band;       // per filter {first bin, bins, offset into fb_w, 0}; an all-zero filter has 0 bins
+    const float *fb_w;         // the bands' weights, packed
+    int fb_n, fb_power;        // filters (1 <= fb_n <= M+1); 1 (|X|) or 2 (|X|^2)
+    float fb_scale, fb_offset, fb_floor;   // L(v) = v if fb_scale == 0, else fb_scale log2(max(v + fb_offset, fb_floor))
 };
-enum { STFT_MODE_DB = 0, STFT_MODE_COMPLEX = 1 };
+enum { STFT_MODE_DB = 0, STFT_MODE_COMPLEX = 1, STFT_MODE_FILTERBANK = 2 };
 // tile -> (signal, tile within the signal) without a division.  Tiles stay below 2^31: each writes at least one row of
 // N/2 + 1 >= 33 floats, and 2^31 such rows are more than device memory holds.
 inline void stft_tile_magic(StftParams &sp) {
@@ -2232,7 +2237,8 @@ __device__ __forceinline__ unsigned stft_tile_signal(long tile, const StftParams
 //   at -100 dB and ten times more per 20 dB deeper.  Everything below the floor (gain - range) clamps to 0 either way, so the error
 //   that counts is the one at the floor; stft_flavour takes the fast form only where it is at most 1e-6 of the
 //   normalised output there, and the exact form below that.
-enum { STFT_K_FAST = 0, STFT_K_EXACT = 1, STFT_K_COMPLEX = 2 };
+// STFT_K_FB (filterbank) writes the per-bin power |X|^p, takes the filter product over it and stores fb_n values per frame.
+enum { STFT_K_FAST = 0, STFT_K_EXACT = 1, STFT_K_COMPLEX = 2, STFT_K_FB = 3 };
 template <int KM> using stft_value_t = typename std::conditional<KM == STFT_K_COMPLEX, float2, float>::type;   // one output bin
 
 __device__ __forceinline__ float stft_db(float re, float im, const StftParams &sp) {
@@ -2262,6 +2268,10 @@ __device__ __forceinline__ void stft_values(const cx<float> (&x)[PL::E], const c
     static_assert(PER * PL::T == HALF, "bins per thread");
     auto conv = [&](int k, cx<R> v) -> V {                               // exact forms (and the three special bins)
         if constexpr (KM == STFT_K_COMPLEX) return make_float2(v.x, v.y);
+        else if constexpr (KM == STFT_K_FB) {                            // |X|^2 or |X|; no bin is zeroed
+            const float p = fmaf(v.x, v.x, v.y * v.y);
+            return sp.fb_power == 2 ? p : sqrtf(p);
+        }
         else return k < 3 ? 0.0f : stft_db(v.x, v.y, sp);               // DC and near-DC bins zeroed (:338-342)
     };
     static_for<PER>([&](auto I_) {
@@ -2292,6 +2302,62 @@ __device__ __forceinline__ void stft_values(const cx<float> (&x)[PL::E], const c
             }
         }
     });
+}
+
+// Filterbank stage (STFT_K_FB).  The per-bin powers of a frame arrive in registers from stft_values; the group writes them
+// as one row of M+1 floats to shared memory and, after a group barrier, each thread computes filters m = tid, tid + T, ...:
+// one f32 FMA chain over the filter's band in increasing bin order, then L.  The same arithmetic on every route, so results
+// are bitwise repeatable and a batch row equals its single-signal run.
+template <class PL, int LAST> struct StftFbValues {
+    static constexpr int PER = PL::E / 2;
+    float vk[PER], vm[PER], vh = 0.0f;
+    __device__ __forceinline__ void take(const cx<float> (&x)[PL::E], const cx<float> *park, const float2 *rtw, int tid,
+                                         const StftParams &sp) {
+        stft_values<PL, LAST, STFT_K_FB>(x, park, rtw, tid, sp, [&](auto I_, int s, int, float v) {
+            CIDX(i, I_);
+            (s == 0 ? vk[i] : s == 1 ? vm[i] : vh) = v;
+        });
+    }
+    __device__ __forceinline__ void to_row(float *row, int tid) const {
+        static_for<PER>([&](auto I_) {
+            CIDX(i, I_);
+            const int k = tid + i * PL::T;
+            row[k] = vk[i];
+            row[PL::N - k] = vm[i];
+            if (i == 0 && k == 0) row[PL::N / 2] = vh;
+        });
+    }
+};
+__device__ __forceinline__ float stft_fb_log(float v, const StftParams &sp) {
+    return sp.fb_scale == 0.0f ? v : sp.fb_scale * __log2f(fmaxf(v + sp.fb_offset, sp.fb_floor));
+}
+// filters m = tid, tid + T, ...: one f32 FMA chain over the band in increasing bin order (float4 loads of weights and
+// powers, and a snake order of filters over threads, were measured slower or no faster: DESIGN §8)
+template <int T, class Out>
+__device__ __forceinline__ void stft_fb_filters(const float *row, int tid, const StftParams &sp, Out &&out) {
+    for (int m = tid; m < sp.fb_n; m += T) {
+        const int4 b = __ldg(sp.fb_band + m);
+        const float *w = sp.fb_w + b.z;
+        const float *p = row + b.x;
+        float acc = 0.0f;
+        for (int j = 0; j < b.y; j++) acc = fmaf(__ldg(w + j), p[j], acc);
+        out(m, stft_fb_log(acc, sp));
+    }
+}
+// direct and pipe kernels: `scratch` is the group's scratch row holding the parked upper half; the results leave from
+// registers.  Every group takes both barriers (groups narrower than a warp share one); only an active one stores.
+template <class PL, int LAST, int X>
+__device__ __forceinline__ void stft_fb_frame(const cx<float> (&x)[PL::E], cx<float> *scratch, const float2 *rtw, int tid, int xi,
+                                              const StftParams &sp, long frame, bool active) {
+    StftFbValues<PL, LAST> v;
+    v.take(x, scratch, rtw, tid, sp);
+    sync_transform<PL::T, X>(xi);                                        // the group has read its parked half
+    float *row = reinterpret_cast<float *>(scratch);
+    v.to_row(row, tid);
+    sync_transform<PL::T, X>(xi);
+    if (!active) return;
+    float *orow = reinterpret_cast<float *>(sp.out) + frame * sp.fb_n;
+    stft_fb_filters<PL::T>(row, tid, sp, [&](int m, float o) { st_stream(orow + m, o); });
 }
 
 // KM: output flavour (STFT_K_*); PAD: window shorter than the FFT size (zero padding)
@@ -2335,6 +2401,10 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft(const __grid_constant__
     if (PL::npass() > 1) sync_transform<PL::T, X>(xi);
     park_upper_half<R, PL, LAST>(x, sm, tid);
     sync_transform<PL::T, X>(xi);
+    if constexpr (KM == STFT_K_FB) {
+        stft_fb_frame<PL, LAST, X>(x, sm, rtw, tid, xi, sp, frame, active);
+        return;
+    }
     if (!active) return;
 
     using V = stft_value_t<KM>;
@@ -2419,7 +2489,8 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_pipe(const __grid_const
         if (PL::npass() > 1) sync_transform<PL::T, X>(xi);
         park_upper_half<R, PL, LAST>(x, scratch, tid);
         sync_transform<PL::T, X>(xi);
-        if (active) {
+        if constexpr (KM == STFT_K_FB) stft_fb_frame<PL, LAST, X>(x, scratch, rtw, tid, xi, sp, frame, active);
+        else if (active) {
             using V = stft_value_t<KM>;
             V *orow = reinterpret_cast<V *>(sp.out) + frame * (M + 1);
             stft_values<PL, LAST, KM>(x, scratch, rtw, tid, sp, [&](auto, int, int bin, V v) { st_stream(orow + bin, v); });
@@ -2502,12 +2573,15 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_span(const __grid_const
         }
     };
     // the result tile of stage `st` sits in `work` at the 16-byte phase of its destination
-    auto out_phase = [&](int st) { return (int)((geom[2 * st] * (long)(M + 1) * VW) & 3); };      // in floats
+    // floats per output row: M+1 bins of VW floats, or one per filter
+    auto row_floats = [&]() -> int { if constexpr (KM == STFT_K_FB) return sp.fb_n; else return (M + 1) * VW; };
+    auto out_phase = [&](int st) { return (int)((geom[2 * st] * (long)row_floats()) & 3); };      // in floats
     auto store_tile = [&](int st) {
         if (threadIdx.x >= 32) return;
-        const long o0 = geom[2 * st] * (long)(M + 1) * VW;               // first float of the tile in the output
-        const int total = tile_rows(geom[2 * st + 1]) * (M + 1) * VW, ph = out_phase(st);
-        const int head = (4 - ph) & 3;                                   // floats up to the next 16-byte boundary
+        const long o0 = geom[2 * st] * (long)row_floats();               // first float of the tile in the output
+        const int total = tile_rows(geom[2 * st + 1]) * row_floats(), ph = out_phase(st);
+        int head = (4 - ph) & 3;                                         // floats up to the next 16-byte boundary
+        if constexpr (KM == STFT_K_FB) head = min(head, total);          // (rows of 1-3 filters: a tile may be shorter)
         const int interior = (total - head) & ~3;
         const float *src = reinterpret_cast<const float *>(work) + ph;
         if (threadIdx.x == 0 && interior > 0) {
@@ -2551,6 +2625,21 @@ __global__ void __launch_bounds__(PL::T *X, MINB) k_stft_span(const __grid_const
         if (PL::npass() > 1) sync_transform<T, X>(xi);
         park_upper_half<R, PL, LAST>(x, scratch, tid);
         sync_transform<T, X>(xi);
+        if constexpr (KM == STFT_K_FB) {
+            // result tile: X rows of fb_n floats at the output's phase; each group's power row of M+1 floats behind it
+            // (fb_n <= M+1, so both fit the complex tile's bytes)
+            StftFbValues<PL, LAST> v;
+            v.take(x, scratch, rtw, tid, sp);
+            __syncthreads();                                             // every group has read its parked half
+            float *row = reinterpret_cast<float *>(work) + 4 + (size_t)X * sp.fb_n + (size_t)xi * (M + 1);
+            v.to_row(row, tid);
+            sync_transform<T, X>(xi);
+            if (geom[2 * st + 1] + xi < sp.frames) {
+                float *orow = reinterpret_cast<float *>(work) + out_phase(st) + (size_t)xi * sp.fb_n;
+                stft_fb_filters<T>(row, tid, sp, [&](int m, float o) { orow[m] = o; });
+            }
+            continue;
+        }
         V vk[PER], vm[PER], vh = V();
         stft_values<PL, LAST, KM>(x, scratch, rtw, tid, sp, [&](auto I_, int s, int, V v) {
             CIDX(i, I_);

@@ -216,21 +216,23 @@ constexpr size_t STFT_SPAN_SMEM_MAX = 200 * 1024;      // the span kernel's shar
 inline size_t stft_span_bytes(int frames, int hop, int wsize) {
     return ((size_t)((long)(frames - 1) * hop + wsize) * sizeof(float) + 127) / 128 * 128;
 }
-// kernel flavour: fast dB / exact dB / complex output.  The fast form drops the +1e-10 of magnitudeToDb, which lowers a
-// value by 20 log10(1 + 1e-10 / (|X| c)) dB, the most at the floor (gain - range): it runs only where that is at most
-// 1e-6 of the [0, 1] output there (floors down to about -99 dB at range 80)
+// kernel flavour: fast dB / exact dB / complex / filterbank output.  The fast form drops the +1e-10 of magnitudeToDb,
+// which lowers a value by 20 log10(1 + 1e-10 / (|X| c)) dB, the most at the floor (gain - range): it runs only where that
+// is at most 1e-6 of the [0, 1] output there (floors down to about -99 dB at range 80)
 inline int stft_flavour(const StftParams &sp) {
     if (sp.mode == STFT_MODE_COMPLEX) return STFT_K_COMPLEX;
+    if (sp.mode == STFT_MODE_FILTERBANK) return STFT_K_FB;
     const double worst = 20.0 * log10(1.0 + 1e-10 * pow(10.0, -(double)sp.db_floor / 20.0)) * (double)sp.inv_range;
     return worst > 1e-6 ? STFT_K_EXACT : STFT_K_FAST;
 }
 // the instantiation k(KM, PAD) of an STFT kernel for a flavour; the unpadded fast-dB case (window = FFT size, the
-// spectrogram default) has its own instantiation without the per-element bound check
+// spectrogram default) has its own instantiation without the per-element bound check; the others exist padded only
 template <class K> const void *stft_kernel(int flavour, bool pad, K k) {
     using std::integral_constant;
     switch (flavour) {
         case STFT_K_FAST: return pad ? k(integral_constant<int, STFT_K_FAST>{}, std::true_type{}) : k(integral_constant<int, STFT_K_FAST>{}, std::false_type{});
         case STFT_K_EXACT: return k(integral_constant<int, STFT_K_EXACT>{}, std::true_type{});
+        case STFT_K_FB: return k(integral_constant<int, STFT_K_FB>{}, std::true_type{});
         default: return k(integral_constant<int, STFT_K_COMPLEX>{}, std::true_type{});
     }
 }
