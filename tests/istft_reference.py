@@ -25,11 +25,8 @@ def istft_reference(spectra, fft_size, hop, window_type="hann", zero_padding=1, 
     if out_len < length:
         raise ValueError("num_samples shorter than the frames reach")
     y = frames_c2r(spectra, fft_size, irfft)
-    num = np.zeros(length)
-    den = np.zeros(length)
-    for f in range(frames):
-        num[f * hop: f * hop + wsize] += w * y[f, :wsize]
-        den[f * hop: f * hop + wsize] += w * w
+    num = overlap_add(w * y[:, :wsize], hop)
+    den = overlap_add(np.broadcast_to(w * w, (frames, wsize)), hop)
     x = np.zeros(out_len)
     ok = den >= 1e-11
     x[:length][ok] = num[ok] / den[ok]
@@ -47,3 +44,11 @@ def frames_c2r(spectra, fft_size, irfft=None):
     z[:, -1] = z[:, -1].real
     return np.fft.irfft(z, fft_size, axis=1)
 
+
+def overlap_add(rows, hop):
+    """sum_f rows[f] placed at sample f*hop, f64, (frames-1)*hop + width samples.  Every sample is summed from 0 in
+    increasing frame order, so the result is bit for bit the per-frame loop `out[f*hop: f*hop + width] += rows[f]`."""
+    rows = np.asarray(rows, np.float64)
+    frames, width = rows.shape
+    idx = (np.arange(frames)[:, None] * hop + np.arange(width)).ravel()
+    return np.bincount(idx, weights=rows.ravel(), minlength=(frames - 1) * hop + width)

@@ -10,7 +10,7 @@ import pytest
 
 import oracle as om
 from conftest import f32_bound
-from istft_reference import frames_c2r, istft_reference
+from istft_reference import frames_c2r, istft_reference, overlap_add
 from stft_reference import stft_f64
 
 WINDOWS = ("hann", "hamming", "blackman", "blackmanHarris", "rectangular")
@@ -23,10 +23,7 @@ def _f32_window(window, wsize):
 def _den(frames, n_fft, hop, window, zp):
     wsize = n_fft // zp
     w = _f32_window(window, wsize)
-    den = np.zeros((frames - 1) * hop + wsize)
-    for f in range(frames):
-        den[f * hop: f * hop + wsize] += w * w
-    return den
+    return overlap_add(np.broadcast_to(w * w, (frames, wsize)), hop)
 
 
 def _bound(spectra, n_fft, hop, window, zp, ref):
@@ -36,9 +33,7 @@ def _bound(spectra, n_fft, hop, window, zp, ref):
     w = np.abs(_f32_window(window, wsize))
     norms = np.linalg.norm(frames_c2r(spectra, n_fft), axis=1)
     frames = spectra.shape[0]
-    acc = np.zeros((frames - 1) * hop + wsize)
-    for f in range(frames):
-        acc[f * hop: f * hop + wsize] += w * (f32_bound(n_fft) * norms[f])
+    acc = overlap_add(w * (f32_bound(n_fft) * norms)[:, None], hop)
     den = _den(frames, n_fft, hop, window, zp)
     out = np.full(len(ref), np.inf)
     ok = den >= 1e-11
